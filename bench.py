@@ -54,7 +54,14 @@ def parse():
                     help="experimental: replay one CUDA graph per optimiser step (actor.cuda_graph_update)")
     ap.add_argument("--rollout", default="auto", choices=["auto", "tc", "fused", "graph"],
                     help="rollout implementation: persistent fused kernel, per-kernel CUDA graph, or the library default")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (see dump_outputs)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return a
 
 
 def workload_name(a):
@@ -441,7 +448,7 @@ def kernel_rooflines(a, peaks, torch):
     bytes_gemm = n * K * 4 + n * 256 * 4
     for key, fn, note in (("tc_gemm_fwd", gemm_all, "C[n,256] = A[n,256] . W^T, plain fp32 in/out; launch includes the 3 us "
                                                     "weight-split kernel of the unit-test entry"),
-                          ("tc_wgrad", wgrad_all, "dW[256,256] += Z[n,256]^T . H[n,256], fp32 atomics into dW")):
+                          ("tc_wgrad", wgrad_all, "dW[256,256] += Z[n,256]^T . H[n,256], per-chunk partials added to dW in a fixed order")):
         t = time_graph(fn, reps_k)
         out[key] = {"bound": "hbm", "achieved": bytes_gemm / t / 1e9, "peak": peaks["hbm_gbs"], "unit": "GB/s",
                     "frac": bytes_gemm / t / 1e9 / peaks["hbm_gbs"],
@@ -461,6 +468,59 @@ def _update_phase_bytes(n, obs, act, H):
     fwd = 2 * (X + U + 2 * U + 2 * U) + 2 * U
     bwd = 4 * U + 2 * (2 * U + 3 * U + 2 * U + 3 * U + (U + X))
     return fwd + bwd
+
+
+DUMP_BYTES = 64 << 20
+DUMP_METRIC_BYTES = 4096  # room kept for the float64 metrics, whose number is known only after the first update
+
+
+def dump_plan(out_dir, run):
+    """The fixed, seeded sample --dump-outputs writes (see dump_outputs), checked against DUMP_BYTES before the benchmark
+    runs: env columns of the [T(+1), B, ...] rollout batch and rows of the [T*B, 1] training batch."""
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    rollout = dict(run.buffer.as_batch())
+    rollout.update(rollout.pop("forward_inputs"))
+    B, T = run.buffer.B, run.buffer.T
+    col_bytes = sum(v[:, 0].numel() * 4 for v in rollout.values())
+    n_cols = max(1, min(B, (DUMP_BYTES // 2) // col_bytes))
+    n_rows = min(T * B, n_cols * T)
+    nbytes = n_cols * col_bytes + 2 * n_rows * 4 + run.actor.model.flat_params.numel() * 4
+    if nbytes + DUMP_METRIC_BYTES > DUMP_BYTES:
+        raise ValueError(f"--dump-outputs: {nbytes} bytes exceed the {DUMP_BYTES}-byte limit at this shape")
+    g = torch.Generator().manual_seed(0)
+    dev = run.buffer.rewards.device
+    cols = torch.randperm(B, generator=g)[:n_cols].sort().values.to(dev)
+    rows = torch.randperm(T * B, generator=g)[:n_rows].sort().values.to(dev)
+    return cols, rows
+
+
+def dump_outputs(out_dir, run, metrics, plan):
+    """Write what the last timed step computed to out_dir/<name>.npy, so that two builds run with the same arguments
+    (hence the same seeded inputs) can be compared output for output:
+      rollout.<key>   the rollout batch the actor consumed ([T(+1), B, ...]), on a fixed, seeded sample of environments
+      train.<key>     advantages / returns of the shuffled training batch ([T*B, 1]), on a fixed, seeded sample of rows
+      param.<name>    every policy parameter after the update
+      metric.<key>    the training metrics the step returned ('/' in a key becomes '.')
+    Float tensors are written as float32, flags as float32 0/1, metrics as float64; at most DUMP_BYTES in all."""
+    import numpy as np
+    import torch
+
+    cols, rows = plan
+    rollout = dict(run.buffer.as_batch())
+    rollout.update(rollout.pop("forward_inputs"))
+    out = {f"rollout.{k}": v.index_select(1, cols) for k, v in rollout.items()}
+    out.update({f"train.{k}": run.actor.rollout_batch[k].index_select(0, rows) for k in ("advantages", "returns")})
+    out.update({f"param.{n}": p for n, p in run.actor.model.named_parameters()})
+    arrays = {k: v.detach().to(torch.float32).cpu().numpy() for k, v in out.items()}
+    arrays.update({f"metric.{k.replace('/', '.')}": np.asarray(v, dtype=np.float64) for k, v in metrics.items()})
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_BYTES}-byte limit at this shape")
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+    log(f"dumped {len(arrays)} arrays ({total / 1e6:.1f} MB) to {out_dir}")
 
 
 def run_ours(a):
@@ -491,6 +551,7 @@ def run_ours(a):
     cfg = synthetic_ppo_config(B=a.B, T=a.T, obs_dim=a.obs, action_dim=a.act, update_epoch=a.update_epoch,
                                num_minibatches=a.minibatches, world_size=world, **over)
     run = EmbodiedRunner(cfg)
+    plan = dump_plan(a.dump_outputs, run) if a.dump_outputs and rank == 0 else None
     n_env_steps = a.B * a.T
 
     def barrier():
@@ -539,6 +600,8 @@ def run_ours(a):
     total_ms = float(t.item())
     ms_per_step = total_ms / a.steps
     value = n_env_steps / (ms_per_step * 1e-3)
+    if a.dump_outputs and rank == 0:  # before the end-to-end steps below move the state on
+        dump_outputs(a.dump_outputs, run, metrics, plan)
 
     # ---- end to end through the public API with HOST buffers (the reference hands the actor CPU tensors) ----
     def pin(d):

@@ -295,7 +295,10 @@ int rb200_mlp_forward(const rb200_mlp_layout* L, const float* params, const floa
                       rb200_stream_t stream);
 
 /* Backward: given d_logprobs [n,act], d_entropy [n,act] or NULL, d_values [n,value_dim] or NULL,
- * ACCUMULATES (+=) parameter gradients into grads (flat, same layout). `acts` from forward. */
+ * ACCUMULATES (+=) parameter gradients into grads (flat, same layout). `acts` from forward.
+ * On the fp16-split tensor-core path (wsplit given, obs_dim % 32 == 0, idx NULL) the sums over rows are stored per
+ * block / sample chunk in `work` and added in a fixed order, so the gradients are bit-identical from run to run;
+ * calls sharing a `work` buffer must be stream-ordered. */
 int rb200_mlp_backward(const rb200_mlp_layout* L, const float* params, const float* wsplit,
                        const float* states, const float* action, const int64_t* idx, int64_t n,
                        const float* d_logprobs, const float* d_entropy, const float* d_values,

@@ -59,6 +59,15 @@ inline cudaStream_t as_stream(rb200_stream_t s) { return reinterpret_cast<cudaSt
 // Per-device scratch (reduction slots); allocated on first use, never freed.
 double* device_scratch(int n_doubles_min);  // defined in abi.cu; returns nullptr on failure
 
+// Cross-block sums without floating-point atomics, so that a result does not depend on the order in which blocks
+// finish: each block stores its partial sums in a row of `part` (stride floats apart), then sum_partials adds the rows
+// in a fixed order.  One segment per output array: out[k] += sum_b part[b * stride + off + k], k < K.
+struct PartialSeg {
+  float* out;
+  int64_t off, K;
+};
+int sum_partials(const float* part, int nparts, int64_t stride, const PartialSeg* segs, int nseg, cudaStream_t st);
+
 inline int sm_count() {
   static int cached[64] = {0};
   int dev = 0;

@@ -187,3 +187,47 @@ extern "C" int rb200_masked_stats(const float* x, const uint8_t* mask, int64_t n
   }
   RB_RETURN_LAUNCH();
 }
+
+namespace rb {
+namespace {
+constexpr int kMaxSegs = 8;
+struct Segs {
+  PartialSeg s[kMaxSegs];
+};
+
+// block = 32 outputs x 32 row phases; grid = (ceil(max K / 32), nseg).  Row phase r sums rows r, r+32, ... in order,
+// then one thread adds the 32 phase sums in order: the same order on every run.
+__global__ void __launch_bounds__(1024) sum_partials_kernel(const float* __restrict__ part, int nparts, int64_t stride,
+                                                            Segs segs) {
+  __shared__ float s[32][33];
+  const PartialSeg g = segs.s[blockIdx.y];
+  const int kx = threadIdx.x & 31, ph = threadIdx.x >> 5;
+  const int64_t k = (int64_t)blockIdx.x * 32 + kx;
+  float acc = 0.f;
+  if (k < g.K)
+    for (int b = ph; b < nparts; b += 32) acc += part[(int64_t)b * stride + g.off + k];
+  s[ph][kx] = acc;
+  __syncthreads();
+  if (ph == 0 && k < g.K) {
+    float t = 0.f;
+#pragma unroll
+    for (int i = 0; i < 32; ++i) t += s[i][kx];
+    g.out[k] += t;
+  }
+}
+}  // namespace
+
+int sum_partials(const float* part, int nparts, int64_t stride, const PartialSeg* segs, int nseg, cudaStream_t st) {
+  if (nseg < 1 || nseg > kMaxSegs || nparts < 1) return RB200_E_SHAPE;
+  Segs S{};
+  int64_t kmax = 0;
+  for (int i = 0; i < nseg; ++i) {
+    S.s[i] = segs[i];
+    if (segs[i].K > kmax) kmax = segs[i].K;
+  }
+  sum_partials_kernel<<<dim3((unsigned)((kmax + 31) / 32), (unsigned)nseg), 1024, 0, st>>>(part, nparts, stride, S);
+  count_launch();
+  cudaError_t ce = cudaPeekAtLastError();
+  return ce == cudaSuccess ? 0 : (int)ce;
+}
+}  // namespace rb

@@ -13,6 +13,8 @@
 // The heads (256 -> act mean, 256 -> value) are fused with the Normal log-prob / entropy epilogue and their backward.
 #include <curand_kernel.h>
 
+#include <algorithm>
+
 #include "common.cuh"
 #include "sgemm.cuh"
 #include "tc_gemm.cuh"
@@ -172,6 +174,7 @@ struct HeadBwdArgs {
   float* g_vb2;             // [256] += column sums of dy3 (value layer 3)
   float* amax_dz3;          // [1] atomicMax |dz3| (operand scaling of the fp16-split gradient GEMMs), or null
   float* amax_dy3;          // [1] atomicMax |dy3|, or null
+  float* part;              // [grid][row] per-block gradient sums (row: see the end of the kernel), added in order by rb::sum_partials
   int64_t n;
   int act, vdim;
 };
@@ -206,6 +209,7 @@ __global__ void __launch_bounds__(256) head_bwd_kernel(HeadBwdArgs p) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = blockDim.x >> 5;
   float cb[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f}, cv[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
   float mz = 0.f, my = 0.f;  // running max |dz3|, |dy3|
+  float rmb = 0.f, rls = 0.f;  // this lane's sums of the mean / log-std gradients (lane < act)
   float rm[REG ? 8 : 1][8], rv[REG ? 2 : 1][8];
 #pragma unroll
   for (int a = 0; a < (REG ? 8 : 1); ++a)
@@ -251,7 +255,11 @@ __global__ void __launch_bounds__(256) head_bwd_kernel(HeadBwdArgs p) {
   const float sd_l = lane < p.act ? expf(p.logstd[lane]) : 1.f;
   const float var_l = sd_l * sd_l;
   RowIn nxt0 = load_row(row_first), nxt1 = load_row(row_first + row_stride);
-  for (int64_t row = row_first; row < p.n; row += row_stride) {
+  // Every warp of the block runs the same number of iterations (the generic path adds into shared memory in warp order at
+  // each one, between barriers); a row past the end loads zeros, contributes zeros and stores nothing.
+  for (int64_t base = (int64_t)blockIdx.x * nwarp; base < p.n; base += row_stride) {
+    const int64_t row = base + warp;
+    const bool live = row < p.n;
     const RowIn cur = nxt0;
     nxt0 = nxt1;
     nxt1 = load_row(row + 2 * row_stride);
@@ -261,8 +269,8 @@ __global__ void __launch_bounds__(256) head_bwd_kernel(HeadBwdArgs p) {
       const float d = cur.x - cur.mu;
       dmu = cur.dlp * d / var_l;
       const float dls = cur.dlp * (d * d / var_l - 1.0f) + cur.den;
-      atomicAdd(&a_mb[lane], dmu);
-      atomicAdd(&a_ls[lane], dls);
+      rmb += dmu;
+      rls += dls;
     }
     float4 dh0 = make_float4(0.f, 0.f, 0.f, 0.f), dh1 = dh0;
 #pragma unroll
@@ -277,21 +285,17 @@ __global__ void __launch_bounds__(256) head_bwd_kernel(HeadBwdArgs p) {
         const int ar = a < 8 ? a : 0;
         rm[ar][0] += g * h0.x; rm[ar][1] += g * h0.y; rm[ar][2] += g * h0.z; rm[ar][3] += g * h0.w;
         rm[ar][4] += g * h1.x; rm[ar][5] += g * h1.y; rm[ar][6] += g * h1.z; rm[ar][7] += g * h1.w;
-        continue;
       }
-      float* am = a_mw + a * kH;
-      atomicAdd(&am[lane * 4 + 0], g * h0.x); atomicAdd(&am[lane * 4 + 1], g * h0.y);
-      atomicAdd(&am[lane * 4 + 2], g * h0.z); atomicAdd(&am[lane * 4 + 3], g * h0.w);
-      atomicAdd(&am[128 + lane * 4 + 0], g * h1.x); atomicAdd(&am[128 + lane * 4 + 1], g * h1.y);
-      atomicAdd(&am[128 + lane * 4 + 2], g * h1.z); atomicAdd(&am[128 + lane * 4 + 3], g * h1.w);
     }
     float4 o0, o1;
     o0.x = dh0.x * (1.f - h0.x * h0.x); o0.y = dh0.y * (1.f - h0.y * h0.y);
     o0.z = dh0.z * (1.f - h0.z * h0.z); o0.w = dh0.w * (1.f - h0.w * h0.w);
     o1.x = dh1.x * (1.f - h1.x * h1.x); o1.y = dh1.y * (1.f - h1.y * h1.y);
     o1.z = dh1.z * (1.f - h1.z * h1.z); o1.w = dh1.w * (1.f - h1.w * h1.w);
-    *reinterpret_cast<float4*>(p.dz3 + row * kH + lane * 4) = o0;
-    *reinterpret_cast<float4*>(p.dz3 + row * kH + 128 + lane * 4) = o1;
+    if (live) {
+      *reinterpret_cast<float4*>(p.dz3 + row * kH + lane * 4) = o0;
+      *reinterpret_cast<float4*>(p.dz3 + row * kH + 128 + lane * 4) = o1;
+    }
     cb[0] += o0.x; cb[1] += o0.y; cb[2] += o0.z; cb[3] += o0.w;
     cb[4] += o1.x; cb[5] += o1.y; cb[6] += o1.z; cb[7] += o1.w;
     mz = fmaxf(mz, fmaxf(fmaxf(fmaxf(fabsf(o0.x), fabsf(o0.y)), fmaxf(fabsf(o0.z), fabsf(o0.w))),
@@ -303,7 +307,7 @@ __global__ void __launch_bounds__(256) head_bwd_kernel(HeadBwdArgs p) {
 #pragma unroll
       for (int c = 0; c < (REG ? 2 : kMaxVal); ++c) {
         if (c >= p.vdim) break;
-        const float g = REG ? (c == 0 ? cur.dv0 : cur.dv1) : p.d_values[row * p.vdim + c];
+        const float g = REG ? (c == 0 ? cur.dv0 : cur.dv1) : (live ? p.d_values[row * p.vdim + c] : 0.f);
         const float4 w0 = *reinterpret_cast<const float4*>(s_vw + c * kH + lane * 4);
         const float4 w1 = *reinterpret_cast<const float4*>(s_vw + c * kH + 128 + lane * 4);
         dg0.x += g * w0.x; dg0.y += g * w0.y; dg0.z += g * w0.z; dg0.w += g * w0.w;
@@ -312,25 +316,46 @@ __global__ void __launch_bounds__(256) head_bwd_kernel(HeadBwdArgs p) {
           const int cr = c < 2 ? c : 0;
           rv[cr][0] += g * g0.x; rv[cr][1] += g * g0.y; rv[cr][2] += g * g0.z; rv[cr][3] += g * g0.w;
           rv[cr][4] += g * g1.x; rv[cr][5] += g * g1.y; rv[cr][6] += g * g1.z; rv[cr][7] += g * g1.w;
-          continue;
         }
-        float* av = a_vw + c * kH;
-        atomicAdd(&av[lane * 4 + 0], g * g0.x); atomicAdd(&av[lane * 4 + 1], g * g0.y);
-        atomicAdd(&av[lane * 4 + 2], g * g0.z); atomicAdd(&av[lane * 4 + 3], g * g0.w);
-        atomicAdd(&av[128 + lane * 4 + 0], g * g1.x); atomicAdd(&av[128 + lane * 4 + 1], g * g1.y);
-        atomicAdd(&av[128 + lane * 4 + 2], g * g1.z); atomicAdd(&av[128 + lane * 4 + 3], g * g1.w);
       }
       float4 q0, q1;
       q0.x = dg0.x * (1.f - g0.x * g0.x); q0.y = dg0.y * (1.f - g0.y * g0.y);
       q0.z = dg0.z * (1.f - g0.z * g0.z); q0.w = dg0.w * (1.f - g0.w * g0.w);
       q1.x = dg1.x * (1.f - g1.x * g1.x); q1.y = dg1.y * (1.f - g1.y * g1.y);
       q1.z = dg1.z * (1.f - g1.z * g1.z); q1.w = dg1.w * (1.f - g1.w * g1.w);
-      *reinterpret_cast<float4*>(p.dy3 + row * kH + lane * 4) = q0;
-      *reinterpret_cast<float4*>(p.dy3 + row * kH + 128 + lane * 4) = q1;
+      if (live) {
+        *reinterpret_cast<float4*>(p.dy3 + row * kH + lane * 4) = q0;
+        *reinterpret_cast<float4*>(p.dy3 + row * kH + 128 + lane * 4) = q1;
+      }
       cv[0] += q0.x; cv[1] += q0.y; cv[2] += q0.z; cv[3] += q0.w;
       cv[4] += q1.x; cv[5] += q1.y; cv[6] += q1.z; cv[7] += q1.w;
       my = fmaxf(my, fmaxf(fmaxf(fmaxf(fabsf(q0.x), fabsf(q0.y)), fmaxf(fabsf(q0.z), fabsf(q0.w))),
                            fmaxf(fmaxf(fabsf(q1.x), fabsf(q1.y)), fmaxf(fabsf(q1.z), fabsf(q1.w)))));
+    }
+    if (!REG) {  // generic path: the warps add this row's weight-gradient terms into shared memory one after another
+      for (int w = 0; w < nwarp; ++w) {
+        if (warp == w) {
+          for (int a = 0; a < p.act; ++a) {
+            const float g = __shfl_sync(0xffffffffu, dmu, a);
+            float* am = a_mw + a * kH;
+            am[lane * 4 + 0] += g * h0.x; am[lane * 4 + 1] += g * h0.y;
+            am[lane * 4 + 2] += g * h0.z; am[lane * 4 + 3] += g * h0.w;
+            am[128 + lane * 4 + 0] += g * h1.x; am[128 + lane * 4 + 1] += g * h1.y;
+            am[128 + lane * 4 + 2] += g * h1.z; am[128 + lane * 4 + 3] += g * h1.w;
+          }
+          if (has_v)
+            for (int c = 0; c < p.vdim; ++c) {
+              const float g = live ? p.d_values[row * p.vdim + c] : 0.f;
+              const float4 g0 = cur.g0, g1 = cur.g1;
+              float* av = a_vw + c * kH;
+              av[lane * 4 + 0] += g * g0.x; av[lane * 4 + 1] += g * g0.y;
+              av[lane * 4 + 2] += g * g0.z; av[lane * 4 + 3] += g * g0.w;
+              av[128 + lane * 4 + 0] += g * g1.x; av[128 + lane * 4 + 1] += g * g1.y;
+              av[128 + lane * 4 + 2] += g * g1.z; av[128 + lane * 4 + 3] += g * g1.w;
+            }
+        }
+        __syncthreads();
+      }
     }
   }
   if (p.amax_dz3 != nullptr) {  // non-negative floats order like their bit patterns
@@ -344,54 +369,54 @@ __global__ void __launch_bounds__(256) head_bwd_kernel(HeadBwdArgs p) {
       if (has_v && my > 0.f && p.amax_dy3) atomicMax(reinterpret_cast<unsigned int*>(p.amax_dy3), __float_as_uint(my));
     }
   }
-  // bias gradients of the two layer-3 pre-activations (lane owns columns lane*4..+3 and 128+lane*4..+3)
-#pragma unroll
-  for (int j = 0; j < 4; ++j) {
-    atomicAdd(&a_b2[lane * 4 + j], cb[j]);
-    atomicAdd(&a_b2[128 + lane * 4 + j], cb[4 + j]);
-    if (has_v) {
-      atomicAdd(&a_vb2[lane * 4 + j], cv[j]);
-      atomicAdd(&a_vb2[128 + lane * 4 + j], cv[4 + j]);
-    }
-  }
-  if (REG) {
-#pragma unroll
-    for (int a = 0; a < 8; ++a) {
-      if (a >= p.act) break;
-      float* am = a_mw + a * kH;
+  // The warps add their register sums into the block's shared sums one after another (warp 0 first): within a warp
+  // every lane owns distinct entries, so the order of every addition is fixed.
+  for (int w = 0; w < nwarp; ++w) {
+    if (warp == w) {
+      if (lane < p.act) {
+        a_mb[lane] += rmb;
+        a_ls[lane] += rls;
+      }
+      // bias gradients of the two layer-3 pre-activations (lane owns columns lane*4..+3 and 128+lane*4..+3)
 #pragma unroll
       for (int j = 0; j < 4; ++j) {
-        atomicAdd(&am[lane * 4 + j], rm[a][j]);
-        atomicAdd(&am[128 + lane * 4 + j], rm[a][4 + j]);
+        a_b2[lane * 4 + j] += cb[j];
+        a_b2[128 + lane * 4 + j] += cb[4 + j];
+        if (has_v) {
+          a_vb2[lane * 4 + j] += cv[j];
+          a_vb2[128 + lane * 4 + j] += cv[4 + j];
+        }
       }
-    }
-    if (has_v) {
+      if (REG) {
 #pragma unroll
-      for (int c = 0; c < 2; ++c) {
-        if (c >= p.vdim) break;
-        float* av = a_vw + c * kH;
+        for (int a = 0; a < 8; ++a) {
+          if (a >= p.act) break;
+          float* am = a_mw + a * kH;
 #pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          atomicAdd(&av[lane * 4 + j], rv[c][j]);
-          atomicAdd(&av[128 + lane * 4 + j], rv[c][4 + j]);
+          for (int j = 0; j < 4; ++j) {
+            am[lane * 4 + j] += rm[a][j];
+            am[128 + lane * 4 + j] += rm[a][4 + j];
+          }
+        }
+        if (has_v) {
+#pragma unroll
+          for (int c = 0; c < 2; ++c) {
+            if (c >= p.vdim) break;
+            float* av = a_vw + c * kH;
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+              av[lane * 4 + j] += rv[c][j];
+              av[128 + lane * 4 + j] += rv[c][4 + j];
+            }
+          }
         }
       }
     }
+    __syncthreads();
   }
-  __syncthreads();
-  for (int i = threadIdx.x; i < p.act * kH; i += blockDim.x)
-    if (a_mw[i] != 0.f) atomicAdd(&p.g_mw[i], a_mw[i]);
-  if (has_v)
-    for (int i = threadIdx.x; i < p.vdim * kH; i += blockDim.x)
-      if (a_vw[i] != 0.f) atomicAdd(&p.g_vw3[i], a_vw[i]);
-  if (threadIdx.x < p.act) {
-    atomicAdd(&p.g_mb[threadIdx.x], a_mb[threadIdx.x]);
-    atomicAdd(&p.g_logstd[threadIdx.x], a_ls[threadIdx.x]);
-  }
-  for (int i = threadIdx.x; i < kH; i += blockDim.x) {
-    atomicAdd(&p.g_b2[i], a_b2[i]);
-    if (has_v) atomicAdd(&p.g_vb2[i], a_vb2[i]);
-  }
+  // the block's sums: one row of the partials buffer, laid out like the shared accumulators from a_mw on
+  const int row_floats = (p.act + p.vdim) * kH + 64 + 2 * kH;
+  for (int i = threadIdx.x; i < row_floats; i += blockDim.x) p.part[(int64_t)blockIdx.x * row_floats + i] = a_mw[i];
 }
 
 int head_grid(int64_t n) {
@@ -514,38 +539,40 @@ int towers_forward_h(const float* X, const int64_t* idx, int64_t n, int in_dim, 
   rb::tch::GemmLaunch g[2];
   if (l0_tc) {
     for (int i = 0; i < nt; ++i) g[i] = rb::tch::GemmLaunch{X, t[i].wh.w0f, nullptr, t[i].H1, t[i].w.b0, nullptr, nullptr, nullptr, nullptr};
-    if ((e = rb::tch::launch(g, nt, n, in_dim, rb::tc::EPI_BIAS_TANH, 0, st))) return e;
+    if ((e = rb::tch::launch(g, nt, n, in_dim, rb::tc::EPI_BIAS_TANH, 0, nullptr, st))) return e;
   } else {
     for (int i = 0; i < nt; ++i)
       if ((e = layer_forward(X, idx, n, in_dim, t[i].w.w0, t[i].w.b0, nullptr, nullptr, t[i].H1, st))) return e;
   }
   for (int i = 0; i < nt; ++i) g[i] = rb::tch::GemmLaunch{t[i].H1, t[i].wh.w1f, nullptr, t[i].H2, t[i].w.b1, nullptr, nullptr, nullptr, nullptr};
-  if ((e = rb::tch::launch(g, nt, n, kH, rb::tc::EPI_BIAS_TANH, 0, st))) return e;
+  if ((e = rb::tch::launch(g, nt, n, kH, rb::tc::EPI_BIAS_TANH, 0, nullptr, st))) return e;
   for (int i = 0; i < nt; ++i) g[i] = rb::tch::GemmLaunch{t[i].H2, t[i].wh.w2f, nullptr, t[i].H3, t[i].w.b2, nullptr, nullptr, nullptr, nullptr};
-  return rb::tch::launch(g, nt, n, kH, rb::tc::EPI_BIAS_TANH, 0, st);
+  return rb::tch::launch(g, nt, n, kH, rb::tc::EPI_BIAS_TANH, 0, nullptr, st);
 }
 
-// backward through the hidden layers of `nt` towers given their dZ3 (and max|dZ3| in amax[0])
-int towers_backward_h(const float* X, const int64_t* idx, int64_t n, int in_dim, TowerIO* t, int nt, cudaStream_t st) {
+// backward through the hidden layers of `nt` towers given their dZ3 (and max|dZ3| in amax[0]); part: partial-sum rows
+// of the gradient GEMMs (part_floats)
+int towers_backward_h(const float* X, const int64_t* idx, int64_t n, int in_dim, TowerIO* t, int nt, float* part,
+                      cudaStream_t st) {
   int e;
   rb::tch::WgradLaunch w[2];
   rb::tch::GemmLaunch g[2];
   // layer 2: dW2 += dZ3^T . H2 ; dZ2 = (dZ3 . W2) * (1 - H2^2)  (+ column sums -> g_b1, max|dZ2| -> amax[1])
   for (int i = 0; i < nt; ++i) w[i] = rb::tch::WgradLaunch{t[i].dZ3, t[i].H2, t[i].g_w2, t[i].amax};
-  if ((e = rb::tch::wgrad(w, nt, n, kH, st))) return e;
+  if ((e = rb::tch::wgrad(w, nt, n, kH, part, st))) return e;
   for (int i = 0; i < nt; ++i)
     g[i] = rb::tch::GemmLaunch{t[i].dZ3, t[i].wh.w2d, nullptr, t[i].tA, nullptr, t[i].H2, t[i].g_b1, t[i].amax, t[i].amax + 1};
-  if ((e = rb::tch::launch(g, nt, n, kH, rb::tc::EPI_TANHGRAD, 1, st))) return e;
+  if ((e = rb::tch::launch(g, nt, n, kH, rb::tc::EPI_TANHGRAD, 1, part, st))) return e;
   // layer 1
   for (int i = 0; i < nt; ++i) w[i] = rb::tch::WgradLaunch{t[i].tA, t[i].H1, t[i].g_w1, t[i].amax + 1};
-  if ((e = rb::tch::wgrad(w, nt, n, kH, st))) return e;
+  if ((e = rb::tch::wgrad(w, nt, n, kH, part, st))) return e;
   for (int i = 0; i < nt; ++i)
     g[i] = rb::tch::GemmLaunch{t[i].tA, t[i].wh.w1d, nullptr, t[i].tB, nullptr, t[i].H1, t[i].g_b0, t[i].amax + 1, t[i].amax + 2};
-  if ((e = rb::tch::launch(g, nt, n, kH, rb::tc::EPI_TANHGRAD, 1, st))) return e;
+  if ((e = rb::tch::launch(g, nt, n, kH, rb::tc::EPI_TANHGRAD, 1, part, st))) return e;
   // layer 0: dW0 += dZ1^T . X
   if (idx == nullptr && (in_dim % rb::tc::BK == 0) && in_dim <= 256) {
     for (int i = 0; i < nt; ++i) w[i] = rb::tch::WgradLaunch{t[i].tB, X, t[i].g_w0, t[i].amax + 2};
-    return rb::tch::wgrad(w, nt, n, in_dim, st);
+    return rb::tch::wgrad(w, nt, n, in_dim, part, st);
   }
   const int64_t rows_per_split = 4096;
   const int splits = (int)((n + rows_per_split - 1) / rows_per_split);
@@ -585,12 +612,26 @@ extern "C" int rb200_mlp_layout_init(rb200_mlp_layout* L, int obs_dim, int act_d
 }
 
 // acts layout (floats): H1 H2 H3 G1 G2 G3, each [n,256] | mean [n,act]
-// work layout: 6 gradient tensors of [n,256]
+// work layout (backward): 6 gradient tensors of [n,256] | 64 floats (max|dZ| slots) | partial-sum rows (part_floats)
 static inline int64_t act_floats(int64_t n) { return n * kH; }
+
+static inline int64_t head_row_floats(const rb200_mlp_layout* L) { return (int64_t)(L->act_dim + L->value_dim) * kH + 64 + 2 * kH; }
+
+// partial-sum rows of one backward: the head kernel's per-block sums, then (reusing the same rows, stream-ordered) the
+// per-chunk / per-CTA sums of the gradient GEMMs
+static int64_t part_floats(const rb200_mlp_layout* L, int64_t n) {
+  int64_t f = (int64_t)head_grid(n) * head_row_floats(L);
+  for (int ng = 1; ng <= 2; ++ng) {
+    f = std::max(f, rb::tch::wgrad_part_floats(ng, n, kH));
+    f = std::max(f, rb::tch::wgrad_part_floats(ng, n, L->obs_dim % rb::tc::BK == 0 && L->obs_dim <= kH ? L->obs_dim : kH));
+    f = std::max(f, rb::tch::launch_part_floats(ng, n));
+  }
+  return f;
+}
 
 extern "C" int64_t rb200_mlp_fwd_scratch_floats(const rb200_mlp_layout* L, int64_t n) {
   if (!L || n <= 0) return 0;
-  return 6 * act_floats(n) + n * L->act_dim + 64;
+  return 6 * act_floats(n) + 64 + std::max(n * L->act_dim, part_floats(L, n));
 }
 
 // wsplit layout (floats), per tower (value tower first, then backbone), every block 16-byte aligned:
@@ -745,6 +786,7 @@ extern "C" int rb200_mlp_backward(const rb200_mlp_layout* L, const float* params
   h.n = n; h.act = L->act_dim; h.vdim = L->value_dim;
   const bool use_h = wsplit && half_mode();
   float* amax = work + 6 * PF;  // 8 floats of the scratch tail: max|dZ3|,|dZ2|,|dZ1| of the policy tower, then the value tower
+  float* part = work + 6 * PF + 64;
   if (use_h) {
     cudaError_t ce = cudaMemsetAsync(amax, 0, 8 * sizeof(float), st);
     if (ce != cudaSuccess) return (int)ce;
@@ -758,14 +800,21 @@ extern "C" int rb200_mlp_backward(const rb200_mlp_layout* L, const float* params
                                           (int)smem);
     if (ce != cudaSuccess) return (int)ce;
   }
+  const int grid = head_grid(n);
+  const int64_t row = head_row_floats(L), va = (int64_t)L->act_dim * kH;
+  h.part = part;
   if (reg)
-    head_bwd_kernel<true><<<head_grid(n), 256, smem, st>>>(h);
+    head_bwd_kernel<true><<<grid, 256, smem, st>>>(h);
   else
-    head_bwd_kernel<false><<<head_grid(n), 256, smem, st>>>(h);
+    head_bwd_kernel<false><<<grid, 256, smem, st>>>(h);
   rb::count_launch();
   {
     cudaError_t ce = cudaPeekAtLastError();
     if (ce != cudaSuccess) return (int)ce;
+    const int64_t o = va + (int64_t)L->value_dim * kH;  // a_mb | a_ls | a_b2 | a_vb2 follow the weight sums
+    rb::PartialSeg segs[6] = {{h.g_mw, 0, va}, {h.g_mb, o, L->act_dim}, {h.g_logstd, o + 32, L->act_dim},
+                              {h.g_b2, o + 64, kH}, {h.g_vw3, va, (int64_t)L->value_dim * kH}, {h.g_vb2, o + 64 + kH, kH}};
+    if ((e = rb::sum_partials(h.part, grid, row, segs, d_values ? 6 : 4, st))) return e;
   }
   if (use_h) {
     TowerIO t[2] = {};
@@ -777,7 +826,7 @@ extern "C" int rb200_mlp_backward(const rb200_mlp_layout* L, const float* params
     t[1].H1 = const_cast<float*>(G1); t[1].H2 = const_cast<float*>(G2); t[1].dZ3 = dY3; t[1].tA = uA; t[1].tB = uB;
     t[1].g_w0 = G + L->vw0; t[1].g_b0 = G + L->vb0; t[1].g_w1 = G + L->vw1; t[1].g_b1 = G + L->vb1;
     t[1].g_w2 = G + L->vw2; t[1].g_b2 = G + L->vb2; t[1].amax = amax + 3;
-    return towers_backward_h(states, idx, n, L->obs_dim, t, d_values ? 2 : 1, st);
+    return towers_backward_h(states, idx, n, L->obs_dim, t, d_values ? 2 : 1, part, st);
   }
   const TowerWS bws = wsplit ? tower_ws(L, wsplit, false) : TowerWS{};
   const TowerWS vws = wsplit ? tower_ws(L, wsplit, true) : TowerWS{};

@@ -69,8 +69,14 @@ struct SplitSpec {
 };
 
 // epi: rb::tc::Epi.  b_mn = 0: C = epi(A . W^T) (forward, W [256,K]);  b_mn = 1: C = epi(A . W) (dgrad, W [256,256]).
-int launch(const GemmLaunch* groups, int ngroups, int64_t M, int K, int epi, int b_mn, cudaStream_t st);
-int wgrad(const WgradLaunch* groups, int ngroups, int64_t n, int IN, cudaStream_t st);
+// The gradient sums of the two launches (dW of wgrad, the column sums of an EPI_TANHGRAD launch with colsum) are stored
+// per sample chunk / CTA in `part` and added by rb::sum_partials in a fixed order: the result does not depend on the order
+// in which CTAs finish.  `part` needs wgrad_part_floats / launch_part_floats floats (launch: may be NULL without colsum);
+// calls sharing it must be stream-ordered.
+int64_t launch_part_floats(int ngroups, int64_t M);
+int64_t wgrad_part_floats(int ngroups, int64_t n, int IN);
+int launch(const GemmLaunch* groups, int ngroups, int64_t M, int K, int epi, int b_mn, float* part, cudaStream_t st);
+int wgrad(const WgradLaunch* groups, int ngroups, int64_t n, int IN, float* part, cudaStream_t st);
 // Weight packs (one launch for all matrices).  Forward pack: k-block kb (32 input features) = the [256 out x 32 k] tile
 // in the K-major SWIZZLE_64B layout, hi (16 KB) then lo (16 KB).  Dgrad pack: k-block kb (32 OUTPUT features = the
 // reduction index of dZ . W) = four [32 out x 64 in] SWIZZLE_128B groups, hi (16 KB) then lo (16 KB).  Both are what

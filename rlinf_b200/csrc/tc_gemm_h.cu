@@ -190,13 +190,13 @@ struct __align__(16) Barriers {
   uint64_t tmem_empty[2];
   uint32_t tmem_base;
   uint32_t pad_[3];
-  alignas(16) float bias[BN];  // (read as float4) forward: the layer bias; dgrad: per-CTA column sums of the output (bias gradient of the producer)
+  alignas(16) float bias[BN];  // (read as float4) forward: the layer bias; dgrad: this CTA's column sums of the output
 };
 
 struct Group {
   const float* bias;    // [256]                         (EPI_BIAS_TANH)
   const float* h;       // [M,256] previous activation   (EPI_TANHGRAD)
-  float* colsum;        // [256] += column sums of the output, or NULL
+  float* colsum;        // [256] += column sums of the output (per-CTA rows of the partials buffer, summed in order), or NULL
   const float* amax_in; // [1] max|A| published by A's producer (gradient GEMMs), or NULL = no scaling
   float* amax_out;      // [1] atomicMax of |output| for the next gradient GEMM, or NULL
 };
@@ -211,6 +211,7 @@ struct GemmParams {
   int b_mn;  // 0: weights K-major (forward), 1: MN-major (dgrad: B(n = in, k = out) = W[out][in])
   int ngroups;
   int flags;
+  float* part;      // [CTAs per group][ngroups][256] column sums (EPI_TANHGRAD with colsum)
   long long* prof;  // [16] (PROF instantiation only)
 };
 
@@ -258,6 +259,9 @@ __global__ void __launch_bounds__(threads_for(kXfWarps), 1) tc_h_gemm_kernel(con
     tmem_relinquish();
   }
   for (int i = threadIdx.x; i < BN; i += kThreads) bars->bias[i] = (P.epi == rb::tc::EPI_BIAS_TANH) ? G.bias[i] : 0.f;
+  // dgrad column sums: each epilogue lane sums its column over the rows of its lane quarter of every tile (csum[i] for
+  // columns c_lo + 32 i + lane); the quarters are added into bars->bias one after another at the end
+  float csum[4] = {0.f, 0.f, 0.f, 0.f};
   fence_before_sync();
   __syncthreads();
   fence_after_sync();
@@ -428,7 +432,7 @@ __global__ void __launch_bounds__(threads_for(kXfWarps), 1) tc_h_gemm_kernel(con
           float cs = 0.f;
 #pragma unroll 8
           for (int rr = 0; rr < 32; ++rr) cs += reinterpret_cast<const float*>(&sh[rr][ch ^ (rr & 7)])[el];
-          atomicAdd(&bars->bias[c0 + lane], cs);
+          csum[(c0 - c_lo) >> 5] += cs;
         }
       }
       fence_before_sync();
@@ -453,9 +457,18 @@ __global__ void __launch_bounds__(threads_for(kXfWarps), 1) tc_h_gemm_kernel(con
   }
   fence_before_sync();
   __syncthreads();
-  if (G.colsum != nullptr && P.epi == rb::tc::EPI_TANHGRAD)
-    for (int i = threadIdx.x; i < BN; i += kThreads)
-      if (bars->bias[i] != 0.f) atomicAdd(G.colsum + i, bars->bias[i]);
+  if (G.colsum != nullptr && P.epi == rb::tc::EPI_TANHGRAD) {
+    const int ew = warp - (2 + kXfWarps);
+    for (int qq = 0; qq < 4; ++qq) {
+      if (ew >= 0 && (warp & 3) == qq) {
+        const int c_lo = (ew >> 2) * (BN / 2);
+#pragma unroll
+        for (int i = 0; i < 4; ++i) bars->bias[c_lo + 32 * i + lane] += csum[i];
+      }
+      __syncthreads();
+    }
+    for (int i = threadIdx.x; i < BN; i += kThreads) P.part[((size_t)cta * P.ngroups + grp) * BN + i] = bars->bias[i];
+  }
   if (warp == 1) {
     fence_after_sync();
     tmem_dealloc(tmem_base, kTmemCols);
@@ -467,7 +480,8 @@ __global__ void __launch_bounds__(threads_for(kXfWarps), 1) tc_h_gemm_kernel(con
 // Per k-block of 32 samples: TMA lands fp32 boxes {32 floats, 32 samples} (SWIZZLE_128B), 8 transform warps split them
 // into fp16 SWIZZLE_64B groups [32 samples x 32 features] = the canonical MN-major SW64 layout with LBO = 2048 B between
 // 32-feature groups and SBO = 512 B between 8-sample atoms; one K=16 MMA step spans two atoms (1024 B).
-// Grid = ngroups x 2 output tiles (128 rows of dW) x sample chunks; fp32 atomics into dW.
+// Grid = ngroups x 2 output tiles (128 rows of dW) x sample chunks; each chunk stores its partial dW in a row of the
+// partials buffer and rb::sum_partials adds the chunks to dW in a fixed order (no float atomics: bit-reproducible).
 // ---------------------------------------------------------------------------------------------------------------
 // Two rings, as in the forward kernel: fp32 landing tiles (dZ 16 KB + H 32 KB per k-block of 32 samples) three deep,
 // freed as soon as the transform has read them, and ONE fp16 operand slot (dZ hi | lo, H hi | lo: 48 KB) that transform
@@ -492,6 +506,7 @@ struct WgBarriers {
 struct WgradParams {
   CUtensorMap z[2], h[2];
   float* dW[2];
+  float* part;             // [chunks][ngroups][256 * IN] partial dW of each sample chunk
   const float* amax_z[2];  // max|dZ| per group (or NULL)
   int64_t n;
   int IN, kb_per_chunk, ngroups, flags;
@@ -589,7 +604,7 @@ __global__ void __launch_bounds__(kWgThreads, 1) tc_h_wgrad_kernel(const __grid_
       fence_after_sync();
       const int row = out_tile * 128 + q * 32 + lane;
       const uint32_t taddr0 = tmem_base + ((uint32_t)(q * 32) << 16);
-      float* dW = P.dW[grp];
+      float* dW = P.part + ((size_t)chunk * P.ngroups + grp) * 256 * IN;
       for (int c0 = 0; c0 < IN; c0 += 32) {
         uint32_t r[32];
         tmem_ld32(taddr0 + c0, r);
@@ -597,9 +612,9 @@ __global__ void __launch_bounds__(kWgThreads, 1) tc_h_wgrad_kernel(const __grid_
         float* dst = dW + (size_t)row * IN + c0;
 #pragma unroll
         for (int j = 0; j < 32; j += 4)
-          atomicAdd(reinterpret_cast<float4*>(dst + j),
-                    make_float4(__uint_as_float(r[j]) * out_scale, __uint_as_float(r[j + 1]) * out_scale,
-                                __uint_as_float(r[j + 2]) * out_scale, __uint_as_float(r[j + 3]) * out_scale));
+          *reinterpret_cast<float4*>(dst + j) =
+              make_float4(__uint_as_float(r[j]) * out_scale, __uint_as_float(r[j + 1]) * out_scale,
+                          __uint_as_float(r[j + 2]) * out_scale, __uint_as_float(r[j + 3]) * out_scale);
       }
       fence_before_sync();
     } else {
@@ -701,14 +716,38 @@ int encode_f16(CUtensorMap* out, const void* base, uint64_t rows, uint64_t cols,
 
 static long long* g_prof = nullptr;  // rb200_tc_h_debug
 
-int launch(const GemmLaunch* L, int ngroups, int64_t M, int K, int epi, int b_mn, cudaStream_t st) {
+static int ctas_per_group(int ngroups, int64_t M) {
+  const int64_t n_tiles = (M + BM - 1) / BM;
+  int per_group = rb::sm_count() / ngroups;
+  if (per_group > n_tiles) per_group = (int)n_tiles;
+  return per_group < 1 ? 1 : per_group;
+}
+
+// sample chunks of the wgrad grid and k-blocks per chunk; every chunk owns at least one k-block (and writes its row)
+static int wgrad_chunks(int ngroups, int64_t n, int* kb_per_chunk) {
+  const int n_kb = (int)((n + BK - 1) / BK);
+  int chunks = rb::sm_count() / (2 * ngroups);
+  if (chunks < 1) chunks = 1;
+  if (chunks > n_kb) chunks = n_kb;
+  *kb_per_chunk = (n_kb + chunks - 1) / chunks;
+  return (n_kb + *kb_per_chunk - 1) / *kb_per_chunk;
+}
+
+int64_t launch_part_floats(int ngroups, int64_t M) { return (int64_t)ctas_per_group(ngroups, M) * ngroups * BN; }
+
+int64_t wgrad_part_floats(int ngroups, int64_t n, int IN) {
+  int kpc = 0;
+  return (int64_t)wgrad_chunks(ngroups, n, &kpc) * ngroups * 256 * IN;
+}
+
+int launch(const GemmLaunch* L, int ngroups, int64_t M, int K, int epi, int b_mn, float* part, cudaStream_t st) {
   if (ngroups < 1 || ngroups > 2 || K % BK != 0 || K <= 0 || M <= 0) return RB200_E_SHAPE;
   // Two towers in one launch: measured on B200 (profiles/r02_tc_h_gemm_grouping.txt) grouped is never slower than one
   // launch per tower (1.18 vs 1.21 ms per 6-GEMM forward at 262144 rows, 0.21 vs 0.24 ms at 32768 where it fills the
   // tail wave).  Debug flag 32 forces one launch per tower.
   if (ngroups == 2 && (rb::tc::g_debug_flags & 32)) {
-    int e = launch(L, 1, M, K, epi, b_mn, st);
-    return e ? e : launch(L + 1, 1, M, K, epi, b_mn, st);
+    int e = launch(L, 1, M, K, epi, b_mn, part, st);
+    return e ? e : launch(L + 1, 1, M, K, epi, b_mn, part, st);
   }
   GemmParams P{};
   P.M = M; P.K = K; P.epi = epi; P.b_mn = b_mn; P.ngroups = ngroups; P.flags = rb::tc::g_debug_flags;
@@ -736,11 +775,16 @@ int launch(const GemmLaunch* L, int ngroups, int64_t M, int K, int epi, int b_mn
     attr_done = true;
   }
   P.prof = g_prof;
-  const int64_t n_tiles = (M + BM - 1) / BM;
-  const int sms = rb::sm_count();
-  int per_group = sms / ngroups;
-  if (per_group > n_tiles) per_group = (int)n_tiles;
-  if (per_group < 1) per_group = 1;
+  const int per_group = ctas_per_group(ngroups, M);
+  rb::PartialSeg segs[2];
+  int nseg = 0;
+  if (epi == rb::tc::EPI_TANHGRAD)
+    for (int g = 0; g < ngroups; ++g)
+      if (L[g].colsum != nullptr) segs[nseg++] = rb::PartialSeg{L[g].colsum, (int64_t)g * BN, BN};
+  if (nseg > 0) {
+    if (part == nullptr) return RB200_E_NULL;
+    P.part = part;
+  }
   // transform warps: 4 (one per scheduler) or 8 (debug flag 64) - see DESIGN.md section 4
   const bool xf8 = ((rb::tc::g_debug_flags & 64) != 0) != (kXfWarpsDefault == 8);
   if (g_prof) tc_h_gemm_kernel<true, 4><<<per_group * ngroups, threads_for(4), kSmem, st>>>(P);
@@ -748,10 +792,11 @@ int launch(const GemmLaunch* L, int ngroups, int64_t M, int K, int epi, int b_mn
   else tc_h_gemm_kernel<false, 4><<<per_group * ngroups, threads_for(4), kSmem, st>>>(P);
   rb::count_launch();
   cudaError_t ce = cudaPeekAtLastError();
-  return ce == cudaSuccess ? 0 : (int)ce;
+  if (ce != cudaSuccess || nseg == 0) return (int)ce;
+  return rb::sum_partials(P.part, per_group, (int64_t)ngroups * BN, segs, nseg, st);
 }
 
-int wgrad(const WgradLaunch* L, int ngroups, int64_t n, int IN, cudaStream_t st) {
+int wgrad(const WgradLaunch* L, int ngroups, int64_t n, int IN, float* part, cudaStream_t st) {
   if (ngroups < 1 || ngroups > 2 || n <= 0 || IN <= 0 || IN > 256 || IN % 32 != 0) return RB200_E_SHAPE;
   WgradParams P{};
   P.n = n; P.IN = IN; P.ngroups = ngroups; P.flags = rb::tc::g_debug_flags;
@@ -775,17 +820,19 @@ int wgrad(const WgradLaunch* L, int ngroups, int64_t n, int IN, cudaStream_t st)
     if (ce != cudaSuccess) return (int)ce;
     attr_done = true;
   }
-  const int n_kb = (int)((n + BK - 1) / BK);
-  int chunks = rb::sm_count() / (2 * ngroups);
-  if (chunks < 1) chunks = 1;
-  if (chunks > n_kb) chunks = n_kb;
-  P.kb_per_chunk = (n_kb + chunks - 1) / chunks;
+  if (part == nullptr) return RB200_E_NULL;
+  const int chunks = wgrad_chunks(ngroups, n, &P.kb_per_chunk);
+  const int64_t stride = (int64_t)ngroups * 256 * IN;
+  P.part = part;
   P.prof = g_prof;
   if (g_prof) tc_h_wgrad_kernel<true><<<ngroups * 2 * chunks, kWgThreads, kSmem, st>>>(P);
   else tc_h_wgrad_kernel<false><<<ngroups * 2 * chunks, kWgThreads, kSmem, st>>>(P);
   rb::count_launch();
   cudaError_t ce = cudaPeekAtLastError();
-  return ce == cudaSuccess ? 0 : (int)ce;
+  if (ce != cudaSuccess) return (int)ce;
+  rb::PartialSeg segs[2];
+  for (int g = 0; g < ngroups; ++g) segs[g] = rb::PartialSeg{L[g].dW, (int64_t)g * 256 * IN, 256ll * IN};
+  return rb::sum_partials(P.part, chunks, stride, segs, ngroups, st);
 }
 
 int split_weights(const SplitSpec* specs, int count, cudaStream_t st) {
@@ -835,12 +882,20 @@ extern "C" int rb200_tc_gemm_h(const float* A, const float* B, float* C, int64_t
   if (e) return e;
   rb::tch::GemmLaunch l{};
   l.a = A; l.b_hi = mode ? sp.lo : sp.hi; l.b_lo = nullptr; l.c = C; l.amax_in = amax;
-  return rb::tch::launch(&l, 1, M, K, rb::tc::EPI_STORE, mode ? 1 : 0, st);
+  return rb::tch::launch(&l, 1, M, K, rb::tc::EPI_STORE, mode ? 1 : 0, nullptr, st);
 }
 
 extern "C" int rb200_tc_wgrad_h(const float* Z, const float* H, float* dW, int64_t n, int IN, const float* amax,
                                 rb200_stream_t stream) {
   if (!Z || !H || !dW) return RB200_E_NULL;
+  if (n <= 0 || IN <= 0 || IN > 256 || IN % 32 != 0) return RB200_E_SHAPE;
+  cudaStream_t st = rb::as_stream(stream);
   rb::tch::WgradLaunch l{Z, H, dW, amax};
-  return rb::tch::wgrad(&l, 1, n, IN, rb::as_stream(stream));
+  // the chunk partials live in a stream-ordered allocation of this call
+  float* part = nullptr;
+  cudaError_t ce = cudaMallocAsync(reinterpret_cast<void**>(&part), sizeof(float) * rb::tch::wgrad_part_floats(1, n, IN), st);
+  if (ce != cudaSuccess) return (int)ce;
+  const int e = rb::tch::wgrad(&l, 1, n, IN, part, st);
+  ce = cudaFreeAsync(part, st);
+  return e ? e : (int)ce;
 }

@@ -406,7 +406,7 @@ def test_two_rank_nccl_update_matches_oracle(tmp_path, graph):
     import sys
 
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     if graph and os.environ.get("RB200_EXPERIMENTAL", "0") != "1":
         # measured on 2 x B200: with the NCCL all-reduce captured inside the step graph the run never completed (500 s
         # timeout, profiles/r02_two_rank_nccl.txt); multi-rank graphed steps are therefore opt-in

@@ -271,7 +271,8 @@ def test_host_batch_e2e_equals_device_batch():
     host = _cpu_batch(a.buffer.as_batch())
     ma = a.update_phase()
     mb = b.update_phase(batch=host)
-    # weight-gradient partial sums use float atomics (order not deterministic): equal to rounding, not bitwise
+    # obs_dim 4 is not a multiple of 32: the first layer's weight gradient goes through the SIMT GEMM, whose per-split
+    # partial sums are added with float atomics (order not deterministic): equal to rounding, not bitwise
     torch.testing.assert_close(a.actor.model.flat_params, b.actor.model.flat_params, rtol=1e-5, atol=1e-7)
     for k in ma:
         np.testing.assert_allclose(ma[k], mb[k], rtol=1e-4, atol=1e-7, err_msg=k)

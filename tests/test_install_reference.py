@@ -1,105 +1,88 @@
-"""INTEGRATION.md's install() against the REAL reference registries (build container only: skipped where
-/root/reference is absent, e.g. on the GPU box).  There is no GPU here, so the check is: every reference entry gets
-replaced, the reference's own dispatchers (`calculate_adv_and_returns`, `policy_loss`, registry.py:77-124) reach the
-replacement with the kwargs its workers build (no TypeError / KeyError on the way), and the replacement then refuses
-to compute on the host (Rb200Error) instead of falling back."""
+"""INTEGRATION.md's install() against the reference's registries, as recorded from the unmodified reference in
+tests/golden/golden_install.npz (tests/golden/make_golden_install.py).  The checks: install() replaces every entry the
+reference registers and accepts every parameter its callables name with the same defaults; the kwargs the reference's
+own dispatchers (`calculate_adv_and_returns`, `policy_loss`, registry.py:77-124) hand the registered callable, for the
+kwargs its workers build, reach the replacement without a TypeError / KeyError, and without a GPU the replacement then
+refuses to compute on the host (Rb200Error) instead of falling back."""
 import inspect
-import os
-import sys
+import json
 
+import numpy as np
 import pytest
 import torch
 
-sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
-import ref_loader  # noqa: E402
 
-pytestmark = pytest.mark.skipif(not ref_loader.reference_available(), reason="reference tree not present")
+def _meta(g):
+    return json.loads(str(g["install_json"]))
 
 
 @pytest.fixture()
-def installed():
-    ref = ref_loader.load_reference()
-    import importlib
+def installed(golden):
+    g = golden("install")
+    meta = _meta(g)
 
-    importlib.import_module("rlinf.algorithms.loss_scales")
-    saved = (dict(ref.registry.ADV_REGISTRY), dict(ref.registry.LOSS_REGISTRY), dict(ref.registry.LOSS_SCALE_REGISTRY))
+    def stand_ins(names):
+        return {name: (lambda name=name: name) for name in names}
+
+    regs = {key: stand_ins(meta["registries"][key]) for key in ("adv", "loss", "loss_scale")}
+    saved = tuple(dict(regs[key]) for key in ("adv", "loss", "loss_scale"))
     import rlinf_b200.plugin as plugin
 
-    done = plugin.install(ref.registry.ADV_REGISTRY, ref.registry.LOSS_REGISTRY, ref.registry.LOSS_SCALE_REGISTRY)
-    yield ref, saved, done
-    for reg, old in zip((ref.registry.ADV_REGISTRY, ref.registry.LOSS_REGISTRY, ref.registry.LOSS_SCALE_REGISTRY), saved):
-        reg.clear()
-        reg.update(old)
+    done = plugin.install(regs["adv"], regs["loss"], regs["loss_scale"])
+    return regs, saved, done, g, meta
 
 
 def test_install_replaces_every_reference_entry(installed):
-    ref, saved, done = installed
+    regs, saved, done, _, meta = installed
     import rlinf_b200.algorithms as A
 
     assert sorted(done["adv"]) == sorted(saved[0]) == sorted(A.ADV_REGISTRY)
     assert sorted(done["loss"]) == sorted(saved[1]) == sorted(A.LOSS_REGISTRY)
     assert sorted(done["loss_scale"]) == sorted(saved[2]) == sorted(A.LOSS_SCALE_REGISTRY)
-    for name, fn in ref.registry.ADV_REGISTRY.items():
+    for name, fn in regs["adv"].items():
         assert fn is A.ADV_REGISTRY[name]
     # signature compatibility: every parameter the reference callable names is accepted by the replacement
-    for old_reg, new_reg in ((saved[0], A.ADV_REGISTRY), (saved[1], A.LOSS_REGISTRY)):
-        for name, old_fn in old_reg.items():
-            old_sig = inspect.signature(inspect.unwrap(old_fn))
+    for key, new_reg in (("adv", A.ADV_REGISTRY), ("loss", A.LOSS_REGISTRY)):
+        for name, old_params in meta["signatures"][key].items():
             new_sig = inspect.signature(new_reg[name])
             new_kw = any(p.kind is inspect.Parameter.VAR_KEYWORD for p in new_sig.parameters.values())
-            for pname, p in old_sig.parameters.items():
-                if p.kind in (inspect.Parameter.VAR_KEYWORD, inspect.Parameter.VAR_POSITIONAL):
+            for p in old_params:
+                pname, default = p["name"], p["default"]
+                if p["kind"] in ("VAR_KEYWORD", "VAR_POSITIONAL"):
                     continue
                 assert pname in new_sig.parameters or new_kw, (name, pname)
                 if pname == "loss_agg_func":
                     continue  # a callable default (masked_mean): the aggregation is selected inside the fused kernel
-                if pname in new_sig.parameters and p.default is not inspect.Parameter.empty:
-                    assert new_sig.parameters[pname].default == p.default, (name, pname)  # same defaults (e.g. A1)
+                assert "callable" not in default, (name, pname)
+                if pname in new_sig.parameters and "value" in default:
+                    assert new_sig.parameters[pname].default == default["value"], (name, pname)  # same defaults (e.g. A1)
 
 
 def test_reference_dispatchers_reach_the_cuda_callables(installed):
-    ref, _, _ = installed
+    regs, _, _, g, meta = installed
     from rlinf_b200._lib import Rb200Error
 
     if torch.cuda.is_available():
-        pytest.skip("build-container check (no GPU): on a GPU box the call would simply succeed")
-    T, B, A = 6, 8, 3
-    g = torch.Generator().manual_seed(0)
-    rewards, values = torch.randn(T, B, 1, generator=g), torch.randn(T + 1, B, 1, generator=g)
-    dones = torch.zeros(T + 1, B, 1, dtype=torch.bool)
-    # kwargs of EmbodiedFSDPActor.compute_advantages_and_returns (embodied_fsdp_actor_worker.py:294-310)
-    adv_kw = dict(task_type="embodied", rewards=rewards, dones=dones, values=values, prev_logprobs=None,
-                  teacher_logprobs=None, num_action_chunks=1, gamma=0.99, gae_lambda=0.95, group_size=4,
-                  reward_type="action_level", loss_mask=None, loss_mask_sum=None, advantage_mode=None)
-    for adv_type in ("gae", "grpo", "raw", "reinpp"):
-        kw = dict(adv_kw, adv_type=adv_type)
-        if adv_type != "gae":
-            lm = torch.ones(T, B, 1, dtype=torch.bool)
-            kw.update(loss_mask=lm, loss_mask_sum=lm.sum(0, keepdim=True).expand_as(lm))
+        pytest.skip("checks the refusal to compute without a GPU: on a GPU the call would simply succeed")
+    kinds = {(c["kind"], c["name"]) for c in meta["calls"]}
+    assert {("adv", t) for t in ("gae", "grpo", "raw", "reinpp")} <= kinds
+    assert {("loss", t) for t in ("actor_critic", "actor", "decoupled_actor_critic")} <= kinds
+    for i, call in enumerate(meta["calls"]):
+        kw = dict(call["scalars"])
+        kw.update({k: torch.from_numpy(np.array(g[f"call_{i}__{k}"])) for k in call["tensors"]})
         with pytest.raises(Rb200Error):
-            ref.registry.calculate_adv_and_returns(**kw)
-    # kwargs of train_micro_batch (:642-676)
-    n = T * B
-    loss_kw = dict(loss_type="actor_critic", logprob_type="action_level", reward_type="action_level", single_action_dim=A,
-                   logprobs=torch.randn(n, A, generator=g), values=torch.randn(n, 1, generator=g),
-                   old_logprobs=torch.randn(n, A, generator=g), advantages=torch.randn(n, 1, generator=g),
-                   returns=torch.randn(n, 1, generator=g), prev_values=torch.randn(n, 1, generator=g), clip_ratio_high=0.2,
-                   clip_ratio_low=0.2, value_clip=0.2, huber_delta=10.0, loss_mask=None, loss_mask_sum=None,
-                   max_episode_steps=80, task_type="embodied", critic_warmup=False)
-    for loss_type in ("actor_critic", "actor", "decoupled_actor_critic"):
-        with pytest.raises(Rb200Error):
-            ref.registry.policy_loss(**dict(loss_kw, loss_type=loss_type))
+            regs[call["kind"]][call["name"]](**kw)
 
 
-def test_logits_wrappers_are_signature_compatible_with_the_reference():
+def test_logits_wrappers_are_signature_compatible_with_the_reference(golden):
     """SURVEY 8(f)3 drop-ins: rlinf_b200.ops.compute_logprobs_from_logits / compute_entropy_from_logits take the reference's
     positional and keyword arguments (rlinf/utils/utils.py:454-512) and, without a GPU, refuse to compute on the host."""
-    ref = ref_loader.load_reference()
+    want_params = _meta(golden("install"))["logits_params"]
     from rlinf_b200 import ops
     from rlinf_b200._lib import Rb200Error
 
     for name in ("compute_logprobs_from_logits", "compute_entropy_from_logits"):
-        want = list(inspect.signature(getattr(ref.utils, name)).parameters)
+        want = want_params[name]
         got = list(inspect.signature(getattr(ops, name)).parameters)
         assert got == want, (name, got, want)
     if not torch.cuda.is_available():
