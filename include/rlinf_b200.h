@@ -453,6 +453,37 @@ int rb200_bootstrap_rewards(float* rewards, const float* final_values, const uin
 int rb200_counter_add(uint64_t* counter_dev, uint64_t inc, rb200_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Policy evaluation (EnvWorker.evaluate / env_evaluate_step, workers/env/env_worker.py:1374-1460, 557-620; episode
+ * bookkeeping of ManiskillEnv, envs/maniskill/maniskill_env.py:232-391; compute_evaluate_metrics,
+ * utils/metric_utils.py:372-420).
+ * ---------------------------------------------------------------------------------------- */
+/* Mean action only: mean [n,act_dim] = actor_mean(backbone(states)) (mode="eval", mlp_policy.py:268-271); no value
+ * tower, no sampling, no log-prob.  Bit-identical to the mean the training head computes.  work: 3*n*256 floats
+ * (rb200_mlp_fwd_scratch_floats(L, n) is enough). */
+int rb200_mlp_mean(const rb200_mlp_layout* L, const float* params, const float* wsplit, const float* states, int64_t n,
+                   float* mean, float* work, rb200_stream_t stream);
+/* One chunk step of the synthetic eval env with per-episode bookkeeping.  Dynamics, noise layout [B, C*(obs+2) + obs]
+ * and Philox streams of rb200_synth_env_step (C = 1) / rb200_synth_env_chunk_step (C > 1), the chunk counter being
+ * `step`; success = the termination draw (u < p_term).  Per sub-step and env: ep_return += r (fp32), success_once |=
+ * success, episode_len = elapsed; ignore_terminations drops the termination after recording.  After the chunk's last
+ * sub-step one record row is written (rec_flags bit 0 = reported: done with auto_reset, else first done since the last
+ * reset; bit 1 = success_once, bit 2 = success_at_end = success of the last sub-step; rec_return, rec_len), then done envs
+ * auto-reset (state from the noise / Philox, elapsed, ep_return and success_once cleared).
+ * state [B,obs] in/out; ep_flags [B] u8 bookkeeping (zero it with elapsed / ep_return at a full reset); scratch 3*B*obs. */
+int rb200_synth_env_eval_step(const float* w_s, const float* w_a, float* state, const float* chunk_actions,
+                              const float* noise, int32_t* elapsed, float* ep_return, uint8_t* ep_flags,
+                              uint8_t* rec_flags, float* rec_return, int32_t* rec_len, float* scratch, int B, int obs,
+                              int act, int C, int max_episode_steps, int auto_reset, int ignore_terminations,
+                              float p_term, float noise_std, float reward_noise_std, uint64_t seed, uint64_t step,
+                              rb200_stream_t stream);
+/* out6 = {sum return, sum episode_len, sum return/episode_len (fp32 quotient), sum success_once, sum success_at_end,
+ * count} over the n records with rec_flags bit 0, accumulated in fp64 in an order that depends on n only (identical
+ * from run to run).  part: RB200_EVAL_MAX_PARTS * 6 doubles of scratch. */
+#define RB200_EVAL_MAX_PARTS 512
+int rb200_eval_metrics(const uint8_t* rec_flags, const float* rec_return, const int32_t* rec_len, int64_t n,
+                       double* part, double* out6, rb200_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------
  * a10 reward filter: replaces the filter_rewards block of EmbodiedFSDPActor._process_received_rollout_batch,
  *   workers/actor/embodied_fsdp_actor_worker.py:236-282 (= preprocess_embodied_batch, rlinf/utils/utils.py:803-830).
  *   rewards f32 [nc,B,C]; loss_mask bool [nc,B,C] or NULL; keep_env bool [B] (scratch/out);

@@ -144,6 +144,10 @@ SIGNATURES = {
     "rb200_kl_penalty": (c_int, [c_void_p] * 4 + [c_int64, c_int, c_void_p]),
     "rb200_masked_stats": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p]),
     "rb200_counter_add": (c_int, [c_void_p, c_uint64, c_void_p]),
+    "rb200_mlp_mean": (c_int, [C.POINTER(MlpLayout), c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p,
+                               c_void_p]),
+    "rb200_synth_env_eval_step": (c_int, [c_void_p] * 12 + [c_int] * 7 + [c_float] * 3 + [c_uint64, c_uint64, c_void_p]),
+    "rb200_eval_metrics": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p]),
     "rb200_masked_moments": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
     "rb200_masked_normalize": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_int, c_double, c_int, c_void_p]),
     "rb200_raw_advantages": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),

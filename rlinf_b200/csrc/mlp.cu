@@ -973,6 +973,59 @@ extern "C" int rb200_mlp_value(const rb200_mlp_layout* L, const float* params, c
   RB_RETURN_LAUNCH();
 }
 
+// actor tower + mean head only (mode="eval": the action is the mean, mlp_policy.py:268-271)
+namespace {
+// the dot products and the bias add of head_fwd_kernel, written the same way so the mean is bit-identical
+__global__ void __launch_bounds__(256) mean_head_kernel(const float* __restrict__ h3, const float* __restrict__ mw,
+                                                        const float* __restrict__ mb, float* __restrict__ mean, int64_t n,
+                                                        int act) {
+  extern __shared__ float s_mw[];  // [act][256]
+  for (int i = threadIdx.x; i < act * kH; i += blockDim.x) s_mw[i] = mw[i];
+  __syncthreads();
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = blockDim.x >> 5;
+  for (int64_t row = (int64_t)blockIdx.x * nwarp + warp; row < n; row += (int64_t)gridDim.x * nwarp) {
+    const float4 h0 = __ldg(reinterpret_cast<const float4*>(h3 + row * kH + lane * 4));
+    const float4 h1 = __ldg(reinterpret_cast<const float4*>(h3 + row * kH + 128 + lane * 4));
+    float my_mean = 0.f;
+    for (int a = 0; a < act; ++a) {
+      const float4 w0 = *reinterpret_cast<const float4*>(s_mw + a * kH + lane * 4);
+      const float4 w1 = *reinterpret_cast<const float4*>(s_mw + a * kH + 128 + lane * 4);
+      float s = h0.x * w0.x + h0.y * w0.y + h0.z * w0.z + h0.w * w0.w + h1.x * w1.x + h1.y * w1.y + h1.z * w1.z +
+                h1.w * w1.w;
+      s = rb::warp_sum(s);
+      if (lane == a) my_mean = s + mb[a];
+    }
+    if (lane < act) mean[row * act + lane] = my_mean;
+  }
+}
+}  // namespace
+
+extern "C" int rb200_mlp_mean(const rb200_mlp_layout* L, const float* params, const float* wsplit, const float* states,
+                              int64_t n, float* mean, float* work, rb200_stream_t stream) {
+  int e = check_layout(L);
+  if (e) return e;
+  if (!params || !states || !mean || !work) return RB200_E_NULL;
+  if (n <= 0) return RB200_E_SHAPE;
+  cudaStream_t st = rb::as_stream(stream);
+  const int64_t PF = act_floats(n);
+  float *H1 = work, *H2 = H1 + PF, *H3 = H2 + PF;
+  if (wsplit && half_mode()) {
+    TowerIO t[1] = {};
+    t[0].w = tower_w(L, params, false); t[0].wh = tower_wh(L, wsplit, false); t[0].H1 = H1; t[0].H2 = H2; t[0].H3 = H3;
+    if ((e = towers_forward_h(states, nullptr, n, L->obs_dim, t, 1, st))) return e;
+  } else {
+    const TowerWS bws = wsplit ? tower_ws(L, wsplit, false) : TowerWS{};
+    if ((e = tower_forward(states, nullptr, n, L->obs_dim, tower_w(L, params, false), wsplit ? &bws : nullptr, H1, H2,
+                           H3, st)))
+      return e;
+  }
+  mean_head_kernel<<<head_grid(n), 256, sizeof(float) * (size_t)L->act_dim * kH, st>>>(H3, params + L->mw,
+                                                                                      params + L->mb, mean, n,
+                                                                                      L->act_dim);
+  rb::count_launch();
+  RB_RETURN_LAUNCH();
+}
+
 // x -> exact-TF32 (hi, lo) pair (hi + lo ~= x to 2^-22). Lets the caller split the shuffled observations once per
 // iteration instead of once per forward call.
 extern "C" int rb200_split_tf32(const float* x, float* hi, float* lo, int64_t n, rb200_stream_t stream) {

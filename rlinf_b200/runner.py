@@ -50,6 +50,12 @@ class EmbodiedRunner:
                                     num_action_chunks=Cn)
         self.rollout = RolloutWorker(cfg, pol, self.env, self.buffer)
         self.global_step = 0
+        self._process_group = process_group
+        self.eval_worker = None  # built on the first evaluate()
+        r = cfg.runner
+        self.max_steps = int(r.max_epochs)  # set_max_steps (embodied_runner.py:655-660): one step per epoch
+        if int(r.get("max_steps", -1)) >= 0:
+            self.max_steps = min(self.max_steps, int(r.max_steps))
         if self.world_size > 1:  # same initial weights everywhere (rank 0's)
             dist.broadcast(pol.flat_params, src=0, group=process_group)
 
@@ -66,6 +72,34 @@ class EmbodiedRunner:
         metrics.update({f"rollout/{k}": v for k, v in rollout_metrics.items()})
         return metrics
 
+    def evaluate(self, return_episodes=False, env_noise=None, init_states=None):
+        """EmbodiedRunner.evaluate (embodied_runner.py:193-206): mean-action episodes on the eval env (`env.eval.*`),
+        aggregated like compute_evaluate_metrics -> {success_once, return, episode_len, reward, [success_at_end],
+        num_trajectories} as floats, over all ranks.  return_episodes: also this rank's per-episode records (eval step
+        major, env index minor).  env_noise / init_states: pre-drawn env noise and initial states (parity tests).
+        Reads the weights the rollout policy holds; call update_rollout_weights() first after an update."""
+        if self.eval_worker is None:
+            from .evaluation import EvalWorker
+
+            self.eval_worker = EvalWorker(self.cfg, self.rollout.policy, self.env, self.rank, self.world_size,
+                                          self._process_group)
+        return self.eval_worker.evaluate(return_episodes, env_noise, init_states)
+
+    def _maybe_eval(self):
+        """_maybe_eval_and_checkpoint (embodied_runner.py:308-329) without checkpointing: evaluate every
+        runner.val_check_interval steps and at the last step, after a weight sync."""
+        r = self.cfg.runner
+        vci = r.get("val_check_interval")
+        if vci is None or vci <= 0:
+            return {}
+        from .evaluation import check_progress
+
+        run_val, _, _ = check_progress(self.global_step, self.max_steps, vci, r.get("save_interval", -1), 1.0)
+        if not run_val:
+            return {}
+        self.update_rollout_weights()
+        return {f"eval/{k}": v for k, v in self.evaluate().items()}
+
     def run_iteration(self):
         self.actor.version = self.global_step
         if self.global_step % self.cfg.runner.get("weight_sync_interval", 1) == 0:
@@ -73,6 +107,7 @@ class EmbodiedRunner:
         self.rollout_phase()
         metrics = self.update_phase()
         self.global_step += 1
+        metrics.update(self._maybe_eval())
         return metrics
 
     def run(self, max_epochs=None):
