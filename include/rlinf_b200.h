@@ -277,18 +277,19 @@ int rb200_mlp_layout_init(rb200_mlp_layout* L, int obs_dim, int act_dim, int val
 /* scratch sizes (floats) for n rows: `acts` and `work` of forward/backward/sample/value each need this many */
 int64_t rb200_mlp_fwd_scratch_floats(const rb200_mlp_layout* L, int64_t n);
 
-/* Tensor-core operand cache: exact-TF32 (hi, lo) copies (and transposes) of the hidden-layer weights.
- * rb200_mlp_wsplit_floats() floats; refresh with rb200_mlp_prepare_weights() after every parameter update.
- * Passing wsplit == NULL to the calls below selects the fp32 SIMT GEMMs for every layer. */
+/* Tensor-core weight cache (`wsplit`, required by the calls below): the hidden-layer weights as packed fp16 (hi, lo)
+ * tiles of w * 2^10, a forward pack per matrix and a dgrad pack per square matrix, in the layout the fp16-split GEMMs
+ * read.  rb200_mlp_wsplit_floats() floats, 16-byte aligned; refresh with rb200_mlp_prepare_weights() after every
+ * parameter update. */
 int64_t rb200_mlp_wsplit_floats(const rb200_mlp_layout* L);
 int rb200_mlp_prepare_weights(const rb200_mlp_layout* L, const float* params, float* wsplit,
                               rb200_stream_t stream);
 
 /* Forward for training: states [n,obs] (row i at idx?idx[i]:i), action [n,act] (same gather).
  * Writes logprobs [n,act], entropy [n,act] (NULL ok), values [n,value_dim] (NULL ok) and keeps
- * the activations needed by backward in `acts`. Hidden layers run on tcgen05 (3xTF32) when wsplit is given
- * and the layer's K is a multiple of 32 (layer 1 additionally needs idx == NULL). Activations are plain fp32; the
- * tensor-core kernels split them into exact-TF32 (hi, lo) operands in shared memory. */
+ * the activations needed by backward in `acts`. Hidden layers run on tcgen05 (kind::f16, 2-way fp16 split, fp32-level
+ * accuracy); the first layer falls back to an fp32 SIMT GEMM when obs_dim % 32 != 0 or idx is given.  Activations are
+ * plain fp32; the tensor-core kernels split them into fp16 (hi, lo) operands in shared memory. */
 int rb200_mlp_forward(const rb200_mlp_layout* L, const float* params, const float* wsplit,
                       const float* states, const float* action, const int64_t* idx, int64_t n,
                       float* logprobs, float* entropy, float* values, float* acts, float* work,
@@ -296,9 +297,10 @@ int rb200_mlp_forward(const rb200_mlp_layout* L, const float* params, const floa
 
 /* Backward: given d_logprobs [n,act], d_entropy [n,act] or NULL, d_values [n,value_dim] or NULL,
  * ACCUMULATES (+=) parameter gradients into grads (flat, same layout). `acts` from forward.
- * On the fp16-split tensor-core path (wsplit given, obs_dim % 32 == 0, idx NULL) the sums over rows are stored per
- * block / sample chunk in `work` and added in a fixed order, so the gradients are bit-identical from run to run;
- * calls sharing a `work` buffer must be stream-ordered. */
+ * The sums over rows are stored per block / sample chunk in `work` and added in a fixed order, so the gradients are
+ * bit-identical from run to run; the exception is the first layer's weight gradient on the fp32 SIMT GEMM (obs_dim % 32
+ * != 0, obs_dim > 256 or idx given), which adds float partial sums with atomics.  Calls sharing a `work` buffer must be
+ * stream-ordered. */
 int rb200_mlp_backward(const rb200_mlp_layout* L, const float* params, const float* wsplit,
                        const float* states, const float* action, const int64_t* idx, int64_t n,
                        const float* d_logprobs, const float* d_entropy, const float* d_values,
@@ -312,33 +314,16 @@ int rb200_mlp_sample(const rb200_mlp_layout* L, const float* params, const float
                      const uint64_t* counter_dev, int64_t n, float* action, float* logprobs, float* values,
                      float* work, rb200_stream_t stream);
 
-/* x[n] -> exact-TF32 pair hi[n], lo[n] with hi + lo ~= x (2^-22 relative): the operand split of the 3xTF32 GEMMs
- * (applied to the weights by rb200_mlp_prepare_weights and, on the fly, to activations inside the GEMM kernels). */
-int rb200_split_tf32(const float* x, float* hi, float* lo, int64_t n, rb200_stream_t stream);
-
-/* 3xTF32 tensor-core GEMM building block of the MLP towers (unit-test entry):
- * C[M,256] = A[M,K] . B[256,K]^T, fp32 in/out, K % 32 == 0; `work` = 512*K floats (split copy of B). */
-int rb200_tc_gemm(const float* A, const float* B, float* C, int64_t M, int K, float* work,
-                  rb200_stream_t stream);
-
-/* Weight-gradient counterpart (unit-test entry): dW[256,IN] += Z[n,256]^T . H[n,IN], IN % 32 == 0, IN <= 256;
- * `work` is unused (may be NULL). */
-int rb200_tc_wgrad(const float* Z, const float* H, float* dW, int64_t n, int IN, float* work,
-                   rb200_stream_t stream);
-/* round 2: the same two unit-test entries for the fp16-split kernel::f16 kernels (csrc/tc_gemm_h.cu).
- * mode 0: C = A[M,K] . B[256,K]^T; mode 1 (dgrad form, K = 256): C = A[M,256] . B[256,256].  amax: device float holding
- * max|A| (or max|Z|), NULL = no operand scaling.  work: >= 512*K floats (packed fp16 weight tiles: forward + dgrad pack). */
+/* Unit-test entries of the fp16-split kind::f16 GEMMs of the MLP towers (csrc/tc_gemm_h.cu), fp32 in/out.
+ * rb200_tc_gemm_h: mode 0: C = A[M,K] . B[256,K]^T; mode 1 (dgrad form, K = 256): C = A[M,256] . B[256,256]; K % 32 == 0;
+ * work: >= 512*K floats (packed fp16 weight tiles: forward + dgrad pack).
+ * rb200_tc_wgrad_h: dW[256,IN] += Z[n,256]^T . H[n,IN], IN % 32 == 0, IN <= 256.
+ * amax: device float holding max|A| (or max|Z|), NULL = no operand scaling. */
 int rb200_tc_gemm_h(const float* A, const float* B, float* C, int64_t M, int K, int mode, const float* amax,
                     float* work, rb200_stream_t stream);
 int rb200_tc_wgrad_h(const float* Z, const float* H, float* dW, int64_t n, int IN, const float* amax,
                      rb200_stream_t stream);
 
-/* Experiment switches (tools/ and tests only; default 0 = the shipped kernels): 1 = additionally mask the streamed operand's
- * hi part in shared memory in the 3xTF32 kernels (not needed: the tensor core truncates), 2 = round-1 layers in the fp32
- * SIMT fused rollout (one-k-step weight prefetch), 8 = round-1 3xTF32 GEMMs instead of the fp16-split ones, 32 = one
- * fp16-split GEMM launch per tower instead of the grouped launch, 64 = 8 transform warps in the fp16-split forward kernel,
- * bits 8-15 = TMA L2-prefetch distance of the 3xTF32 kernels in k-blocks (255 = off). */
-int rb200_debug_set_flags(int flags);
 /* probe hook of the fp16-split GEMM (csrc/tc_gemm_h.cu): 16 int64 per-role wait / work cycle counters of CTA 0 */
 int rb200_tc_h_debug(void* prof16);
 

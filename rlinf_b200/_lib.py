@@ -112,13 +112,9 @@ SIGNATURES = {
     "rb200_mlp_prepare_weights": (c_int, [C.POINTER(MlpLayout), c_void_p, c_void_p, c_void_p]),
     "rb200_mlp_forward": (c_int, [C.POINTER(MlpLayout)] + [c_void_p] * 5 + [c_int64] + [c_void_p] * 6),
     "rb200_mlp_backward": (c_int, [C.POINTER(MlpLayout)] + [c_void_p] * 5 + [c_int64] + [c_void_p] * 7),
-    "rb200_split_tf32": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p]),
     "rb200_mlp_sample": (c_int, [C.POINTER(MlpLayout)] + [c_void_p] * 4 + [c_uint64, c_uint64, c_void_p, c_int64] + [c_void_p] * 5),
-    "rb200_tc_gemm": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p]),
-    "rb200_tc_wgrad": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p]),
     "rb200_tc_gemm_h": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int, c_void_p, c_void_p, c_void_p]),
     "rb200_tc_wgrad_h": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int, c_void_p, c_void_p]),
-    "rb200_debug_set_flags": (c_int, [c_int]),
     "rb200_tc_h_debug": (c_int, [c_void_p]),
     "rb200_rollout_fused_wt_floats": (c_int64, [C.POINTER(MlpLayout)]),
     "rb200_rollout_fused_supported": (c_int, [C.POINTER(MlpLayout), c_int]),

@@ -4,12 +4,12 @@
 // ValueHead, rlinf/models/embodiment/modules/value_head.py:18-67 (3x256 tanh MLP -> value_dim, last layer
 // without bias); backward = what autograd derives from them.
 //
-// Hidden-layer GEMMs run on the tensor cores whenever the operand shapes allow TMA (K % 32 == 0, no row gather): by
-// default the fp16-split kernels (tc_gemm_h.cu: tcgen05 kind::f16, a = a_hi + a_lo in fp16, three MMAs per product,
-// fp32-level accuracy, both towers per launch), with debug flag 8 the round-1 3xTF32 kernels (tc_gemm.cu); the fp32 SIMT
-// GEMM (sgemm.cuh) covers the remaining shapes.  Activations and activation-gradients are stored once, as plain fp32
-// [n,256] (6 tanh outputs per forward, tanh' = 1 - h^2); the tensor-core kernels split them into (hi, lo) pairs on the
-// fly in shared memory.
+// Hidden-layer GEMMs run on the fp16-split tensor-core kernels (tc_gemm_h.cu: tcgen05 kind::f16, a = a_hi + a_lo in fp16,
+// three MMAs per product, fp32-level accuracy, both towers per launch), reading the weights from the packs that
+// rb200_mlp_prepare_weights writes into the caller's wsplit buffer.  Layer 0 falls back to the fp32 SIMT GEMM (sgemm.cuh)
+// when its operand cannot be TMA-tiled (obs_dim % 32 != 0, or rows gathered through idx; for its weight gradient also
+// obs_dim > 256).  Activations and activation-gradients are stored once, as plain fp32 [n,256] (6 tanh outputs per
+// forward, tanh' = 1 - h^2); the tensor-core kernels split them into (hi, lo) pairs on the fly in shared memory.
 // The heads (256 -> act mean, 256 -> value) are fused with the Normal log-prob / entropy epilogue and their backward.
 #include <curand_kernel.h>
 
@@ -22,25 +22,6 @@
 namespace {
 
 using namespace rb::gemm;
-
-// out[n] += sum_m Z[m][n]   (bias gradients); Z is [M, N] with N <= 1024
-__global__ void __launch_bounds__(256) colsum_kernel(const float* __restrict__ Z, float* __restrict__ out, int64_t M, int N,
-                                                     int64_t rows_per_block) {
-  const int64_t r0 = (int64_t)blockIdx.x * rows_per_block;
-  const int64_t r1 = (r0 + rows_per_block < M) ? r0 + rows_per_block : M;
-  for (int n = threadIdx.x; n < N; n += blockDim.x) {
-    float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
-    int64_t r = r0;
-    for (; r + 3 < r1; r += 4) {
-      s0 += Z[r * N + n];
-      s1 += Z[(r + 1) * N + n];
-      s2 += Z[(r + 2) * N + n];
-      s3 += Z[(r + 3) * N + n];
-    }
-    for (; r < r1; ++r) s0 += Z[r * N + n];
-    atomicAdd(&out[n], (s0 + s1) + (s2 + s3));
-  }
-}
 
 // ------------------------------------------------------------------------------------------------
 // Fused heads.  One warp per sample row; H = 256 hidden units -> 8 per lane (two float4).
@@ -429,93 +410,18 @@ int head_grid(int64_t n) {
 // ---------------------------------------------------------------------------------------------------------
 // Towers.  Activation / gradient tensors are plain fp32 [n,256].
 // ---------------------------------------------------------------------------------------------------------
-struct TowerW {           // fp32 weights (SIMT path)
+struct TowerW {           // fp32 weights and biases as stored in the parameters
   const float *w0, *b0, *w1, *b1, *w2, *b2;
 };
-struct TowerWS {          // exact-TF32 (hi, lo) copies for the tensor cores (null => SIMT everywhere)
-  const float *w0h, *w0l, *w1h, *w1l, *w2h, *w2l;   // [256,in] as stored (forward:  X . W^T)
-  const float *w1th, *w1tl, *w2th, *w2tl;           // transposed [in=256, out=256] (dgrad: dZ . W)
-};
 
-// one hidden layer forward: out = tanh(in . W^T + b)
+// one hidden layer forward on the SIMT GEMM: out = tanh(in . W^T + b)
 int layer_forward(const float* in, const int64_t* idx, int64_t n, int in_dim, const float* w, const float* b,
-                  const float* wh, const float* wl, float* out, cudaStream_t st) {
-  const bool tc_ok = wh != nullptr && idx == nullptr && (in_dim % rb::tc::BK == 0);
-  if (tc_ok) {
-    rb::tc::Params p{};
-    p.M = n; p.K = in_dim; p.bias = b; p.c = out; p.epi = rb::tc::EPI_BIAS_TANH;
-    return rb::tc::launch(in, wh, wl, p, st);
-  }
+                  float* out, cudaStream_t st) {
   GemmArgs g{};
   g.M = n; g.N = kH; g.ldc = kH; g.k_per_split = 1 << 30;
   g.A = in; g.lda = in_dim; g.a_rows = idx; g.B = w; g.ldb = in_dim; g.K = in_dim; g.bias = b; g.C = out;
   return launch_gemm<A_KCONTIG, B_KCONTIG, EPI_BIAS_TANH>(g, 1, st);
 }
-
-// X -> H1 -> H2 -> H3 (each [n,256])
-int tower_forward(const float* X, const int64_t* idx, int64_t n, int in_dim, const TowerW& w, const TowerWS* ws,
-                  float* H1, float* H2, float* H3, cudaStream_t st) {
-  int e = layer_forward(X, idx, n, in_dim, w.w0, w.b0, ws ? ws->w0h : nullptr, ws ? ws->w0l : nullptr, H1, st);
-  if (e) return e;
-  e = layer_forward(H1, nullptr, n, kH, w.w1, w.b1, ws ? ws->w1h : nullptr, ws ? ws->w1l : nullptr, H2, st);
-  if (e) return e;
-  return layer_forward(H2, nullptr, n, kH, w.w2, w.b2, ws ? ws->w2h : nullptr, ws ? ws->w2l : nullptr, H3, st);
-}
-
-// backward through the three hidden layers of one tower, given dZ3. tmpA/tmpB: [n,256] scratch.
-int tower_backward(const float* X, const int64_t* idx, int64_t n, int in_dim, const TowerW& w, const TowerWS* ws,
-                   const float* H1, const float* H2, const float* dZ3, float* tmpA, float* tmpB, float* g_w0,
-                   float* g_b0, float* g_w1, float* g_b1, float* g_w2, float* g_b2, cudaStream_t st) {
-  const int64_t rows_per_split = 4096;
-  const int splits = (int)((n + rows_per_split - 1) / rows_per_split);
-  const int64_t cs_rows = 128;
-  const int cs_blocks = (int)((n + cs_rows - 1) / cs_rows);
-  int e;
-  auto colsum = [&](const float* dZ, float* gb) -> int {
-    colsum_kernel<<<cs_blocks, 256, 0, st>>>(dZ, gb, n, kH, cs_rows);
-    rb::count_launch();
-    cudaError_t ce = cudaPeekAtLastError();
-    return ce == cudaSuccess ? 0 : (int)ce;
-  };
-  auto wgrad = [&](const float* dZ, const float* Hin, const int64_t* in_rows, int in_ld, float* gw, float* gb,
-                   bool need_colsum) -> int {
-    // gw[256, in_ld] += dZ^T [256, n] . Hin [n, in_ld]
-    int ee;
-    if (ws && !in_rows && (in_ld % rb::tc::BK == 0) && in_ld <= 256) {  // tensor cores (3xTF32)
-      ee = rb::tc::wgrad(dZ, Hin, gw, n, in_ld, st);
-    } else {  // fp32 SIMT, split over samples, atomics
-      GemmArgs g{};
-      g.A = dZ; g.lda = kH; g.B = Hin; g.ldb = in_ld; g.b_rows = in_rows; g.C = gw;
-      g.ldc = in_ld; g.M = kH; g.N = in_ld; g.K = n; g.k_per_split = rows_per_split;
-      ee = launch_gemm<A_MCONTIG, B_NCONTIG, EPI_ATOMIC>(g, splits, st);
-    }
-    if (ee || !need_colsum) return ee;
-    return colsum(dZ, gb);
-  };
-  auto dgrad = [&](const float* dZ, const float* W, const float* Wth, const float* Wtl, const float* Hprev,
-                   float* out, float* gb_prev) -> int {
-    // out = (dZ . W) * (1 - Hprev^2); the tensor-core epilogue also adds out's column sums to gb_prev
-    if (Wth) {
-      rb::tc::Params p{};
-      p.M = n; p.K = kH; p.h = Hprev; p.c = out; p.colsum = gb_prev; p.epi = rb::tc::EPI_TANHGRAD;
-      return rb::tc::launch(dZ, Wth, Wtl, p, st);
-    }
-    GemmArgs g{};
-    g.A = dZ; g.lda = kH; g.B = W; g.ldb = kH; g.C = out; g.ldc = kH; g.aux = Hprev;
-    g.ldaux = kH; g.M = n; g.N = kH; g.K = kH; g.k_per_split = 1 << 30;
-    return launch_gemm<A_KCONTIG, B_NCONTIG, EPI_TANHGRAD>(g, 1, st);
-  };
-  const bool tc = ws != nullptr;  // tensor-core dgrad adds the bias gradients of layers 2 and 1 in its epilogue
-  if ((e = wgrad(dZ3, H2, nullptr, kH, g_w2, g_b2, false))) return e;  // g_b2: head_bwd_kernel
-  if ((e = dgrad(dZ3, w.w2, ws ? ws->w2th : nullptr, ws ? ws->w2tl : nullptr, H2, tmpA, g_b1))) return e;  // dZ2
-  if ((e = wgrad(tmpA, H1, nullptr, kH, g_w1, g_b1, !tc))) return e;
-  if ((e = dgrad(tmpA, w.w1, ws ? ws->w1th : nullptr, ws ? ws->w1tl : nullptr, H1, tmpB, g_b0))) return e;  // dZ1
-  return wgrad(tmpB, X, idx, in_dim, g_w0, g_b0, !tc);
-}
-
-// ---- round 2: fp16-split tensor-core path (tc_gemm_h.cu), both towers per launch -------------------------------------------
-// debug flag bit 3 (value 8) selects the round-1 3xTF32 kernels instead.
-inline bool half_mode() { return (rb::tc::g_debug_flags & 8) == 0; }
 
 struct TowerWH {  // packed fp16 (hi, lo) tiles of w * 2^10 (rb::tch::split_weights); typed float* (they live in the wsplit buffer)
   const float *w0f, *w1f, *w2f;  // forward packs of layers 0..2
@@ -542,7 +448,7 @@ int towers_forward_h(const float* X, const int64_t* idx, int64_t n, int in_dim, 
     if ((e = rb::tch::launch(g, nt, n, in_dim, rb::tc::EPI_BIAS_TANH, 0, nullptr, st))) return e;
   } else {
     for (int i = 0; i < nt; ++i)
-      if ((e = layer_forward(X, idx, n, in_dim, t[i].w.w0, t[i].w.b0, nullptr, nullptr, t[i].H1, st))) return e;
+      if ((e = layer_forward(X, idx, n, in_dim, t[i].w.w0, t[i].w.b0, t[i].H1, st))) return e;
   }
   for (int i = 0; i < nt; ++i) g[i] = rb::tch::GemmLaunch{t[i].H1, t[i].wh.w1f, nullptr, t[i].H2, t[i].w.b1, nullptr, nullptr, nullptr, nullptr};
   if ((e = rb::tch::launch(g, nt, n, kH, rb::tc::EPI_BIAS_TANH, 0, nullptr, st))) return e;
@@ -634,9 +540,9 @@ extern "C" int64_t rb200_mlp_fwd_scratch_floats(const rb200_mlp_layout* L, int64
   return 6 * act_floats(n) + 64 + std::max(n * L->act_dim, part_floats(L, n));
 }
 
-// wsplit layout (floats), per tower (value tower first, then backbone), every block 16-byte aligned:
-//   w0h w0l [256*obs] | w1h w1l w2h w2l [65536 each] | w1th w1tl w2th w2tl [65536 each]
-static inline int64_t wsplit_tower_floats(int obs) { return 2ll * kH * obs + 8ll * kH * kH; }
+// wsplit layout, per tower (value tower first, then backbone): packed fp16 (hi, lo) tiles (rb::tch::split_weights), one
+// float of storage per weight: forward packs of w0 [256*obs], w1, w2 [65536 each], then the dgrad packs of w1, w2
+static inline int64_t wsplit_tower_floats(int obs) { return (int64_t)kH * obs + 4ll * kH * kH; }
 
 extern "C" int64_t rb200_mlp_wsplit_floats(const rb200_mlp_layout* L) {
   if (!L) return 0;
@@ -660,22 +566,9 @@ TowerW tower_w(const rb200_mlp_layout* L, const float* P, bool value) {
   }
   return w;
 }
-TowerWS tower_ws(const rb200_mlp_layout* L, const float* ws, bool value) {
-  const float* b = ws + (value ? 0 : wsplit_tower_floats(L->obs_dim));
-  const int64_t n0 = (int64_t)kH * L->obs_dim, nn = (int64_t)kH * kH;
-  TowerWS t;
-  t.w0h = b; t.w0l = b + n0;
-  const float* q = b + 2 * n0;
-  t.w1h = q; t.w1l = q + nn; t.w2h = q + 2 * nn; t.w2l = q + 3 * nn;
-  t.w1th = q + 4 * nn; t.w1tl = q + 5 * nn; t.w2th = q + 6 * nn; t.w2tl = q + 7 * nn;
-  return t;
-}
-// fp16-split cache, per tower (value tower first): forward packs of w0 [256*obs floats of storage], w1, w2 [65536 each],
-// then the dgrad packs of w1, w2; it needs less than the TF32 cache, so it lives in the same buffer
 TowerWH tower_wh(const rb200_mlp_layout* L, const float* ws, bool value) {
-  const int64_t n0 = (int64_t)kH * L->obs_dim, nn = (int64_t)kH * kH;  // floats of storage (4 bytes per element: hi + lo)
-  const int64_t per_tower = n0 + 4 * nn;
-  const float* b = ws + (value ? 0 : per_tower);
+  const int64_t n0 = (int64_t)kH * L->obs_dim, nn = (int64_t)kH * kH;
+  const float* b = ws + (value ? 0 : wsplit_tower_floats(L->obs_dim));
   TowerWH t;
   t.w0f = b;
   t.w1f = b + n0;
@@ -686,42 +579,26 @@ TowerWH tower_wh(const rb200_mlp_layout* L, const float* ws, bool value) {
 }
 }  // namespace
 
-// Refresh the weight copies the tensor-core GEMMs read: packed fp16 (hi, lo) tiles in ONE launch (default), or the
-// exact-TF32 (hi, lo) copies of the round-1 kernels (debug flag 8; 2 x 10 tiny kernels). Call after every parameter update
-// (once per optimiser step / once per rollout).
+// Refresh the weight packs the tensor-core GEMMs read: fp16 (hi, lo) of w * 2^10 for all hidden matrices in ONE launch.
+// Call after every parameter update (once per optimiser step / once per rollout).
 extern "C" int rb200_mlp_prepare_weights(const rb200_mlp_layout* L, const float* params, float* wsplit,
                                          rb200_stream_t stream) {
   int e = check_layout(L);
   if (e) return e;
   if (!params || !wsplit) return RB200_E_NULL;
-  cudaStream_t st = rb::as_stream(stream);
-  if (half_mode()) {  // fp16 (hi, lo) of w * 2^10 for all hidden matrices: ONE launch (round 1: 20 kernels)
-    rb::tch::SplitSpec sp[6];
-    int cnt = 0;
-    for (int v = 0; v < 2; ++v) {
-      if (v == 0 && L->value_dim == 0) continue;
-      const TowerW w = tower_w(L, params, v == 0);
-      const TowerWH t = tower_wh(L, wsplit, v == 0);
-      const int64_t n0 = (int64_t)kH * L->obs_dim, nn = (int64_t)kH * kH;
-      if (L->obs_dim % rb::tc::BK == 0)  // layer 0 runs on the tensor cores only then
-        sp[cnt++] = rb::tch::SplitSpec{w.w0, const_cast<float*>(t.w0f), nullptr, n0};
-      sp[cnt++] = rb::tch::SplitSpec{w.w1, const_cast<float*>(t.w1f), const_cast<float*>(t.w1d), nn};
-      sp[cnt++] = rb::tch::SplitSpec{w.w2, const_cast<float*>(t.w2f), const_cast<float*>(t.w2d), nn};
-    }
-    return rb::tch::split_weights(sp, cnt, st);
-  }
+  rb::tch::SplitSpec sp[6];
+  int cnt = 0;
   for (int v = 0; v < 2; ++v) {
     if (v == 0 && L->value_dim == 0) continue;
     const TowerW w = tower_w(L, params, v == 0);
-    const TowerWS t = tower_ws(L, wsplit, v == 0);
+    const TowerWH t = tower_wh(L, wsplit, v == 0);
     const int64_t n0 = (int64_t)kH * L->obs_dim, nn = (int64_t)kH * kH;
-    if ((e = rb::tc::split(w.w0, const_cast<float*>(t.w0h), const_cast<float*>(t.w0l), n0, st))) return e;
-    if ((e = rb::tc::split(w.w1, const_cast<float*>(t.w1h), const_cast<float*>(t.w1l), nn, st))) return e;
-    if ((e = rb::tc::split(w.w2, const_cast<float*>(t.w2h), const_cast<float*>(t.w2l), nn, st))) return e;
-    if ((e = rb::tc::split_transpose(w.w1, const_cast<float*>(t.w1th), const_cast<float*>(t.w1tl), kH, kH, st))) return e;
-    if ((e = rb::tc::split_transpose(w.w2, const_cast<float*>(t.w2th), const_cast<float*>(t.w2tl), kH, kH, st))) return e;
+    if (L->obs_dim % rb::tc::BK == 0)  // layer 0 runs on the tensor cores only then
+      sp[cnt++] = rb::tch::SplitSpec{w.w0, const_cast<float*>(t.w0f), nullptr, n0};
+    sp[cnt++] = rb::tch::SplitSpec{w.w1, const_cast<float*>(t.w1f), const_cast<float*>(t.w1d), nn};
+    sp[cnt++] = rb::tch::SplitSpec{w.w2, const_cast<float*>(t.w2f), const_cast<float*>(t.w2d), nn};
   }
-  return RB200_OK;
+  return rb::tch::split_weights(sp, cnt, rb::as_stream(stream));
 }
 
 extern "C" int rb200_mlp_forward(const rb200_mlp_layout* L, const float* params, const float* wsplit,
@@ -730,7 +607,7 @@ extern "C" int rb200_mlp_forward(const rb200_mlp_layout* L, const float* params,
                                  rb200_stream_t stream) {
   int e = check_layout(L);
   if (e) return e;
-  if (!params || !states || !action || !logprobs || !acts || !work) return RB200_E_NULL;
+  if (!params || !wsplit || !states || !action || !logprobs || !acts || !work) return RB200_E_NULL;
   if (n <= 0) return RB200_E_SHAPE;
   if (values && L->value_dim == 0) return RB200_E_SHAPE;
   cudaStream_t st = rb::as_stream(stream);
@@ -738,20 +615,10 @@ extern "C" int rb200_mlp_forward(const rb200_mlp_layout* L, const float* params,
   float *H1 = acts, *H2 = H1 + PF, *H3 = H2 + PF, *G1 = H3 + PF, *G2 = G1 + PF, *G3 = G2 + PF;
   float* mean = G3 + PF;
   const float* P = params;
-  const TowerWS bws = wsplit ? tower_ws(L, wsplit, false) : TowerWS{};
-  const TowerWS vws = wsplit ? tower_ws(L, wsplit, true) : TowerWS{};
-  if (wsplit && half_mode()) {
-    TowerIO t[2] = {};
-    t[0].w = tower_w(L, P, false); t[0].wh = tower_wh(L, wsplit, false); t[0].H1 = H1; t[0].H2 = H2; t[0].H3 = H3;
-    t[1].w = tower_w(L, P, true);  t[1].wh = tower_wh(L, wsplit, true);  t[1].H1 = G1; t[1].H2 = G2; t[1].H3 = G3;
-    if ((e = towers_forward_h(states, idx, n, L->obs_dim, t, values ? 2 : 1, st))) return e;
-  } else {
-    if ((e = tower_forward(states, idx, n, L->obs_dim, tower_w(L, P, false), wsplit ? &bws : nullptr, H1, H2, H3, st)))
-      return e;
-    if (values &&
-        (e = tower_forward(states, idx, n, L->obs_dim, tower_w(L, P, true), wsplit ? &vws : nullptr, G1, G2, G3, st)))
-      return e;
-  }
+  TowerIO t[2] = {};
+  t[0].w = tower_w(L, P, false); t[0].wh = tower_wh(L, wsplit, false); t[0].H1 = H1; t[0].H2 = H2; t[0].H3 = H3;
+  t[1].w = tower_w(L, P, true);  t[1].wh = tower_wh(L, wsplit, true);  t[1].H1 = G1; t[1].H2 = G2; t[1].H3 = G3;
+  if ((e = towers_forward_h(states, idx, n, L->obs_dim, t, values ? 2 : 1, st))) return e;
   HeadFwdArgs h{};
   h.h3 = H3; h.g3 = values ? G3 : nullptr; h.mw = P + L->mw; h.mb = P + L->mb;
   h.logstd = P + L->logstd; h.vw3 = P + L->vw3; h.action = action; h.idx = idx; h.sample_mode = 0; h.mean_out = mean;
@@ -768,7 +635,7 @@ extern "C" int rb200_mlp_backward(const rb200_mlp_layout* L, const float* params
                                   const float* acts, float* work, float* grads, rb200_stream_t stream) {
   int e = check_layout(L);
   if (e) return e;
-  if (!params || !states || !action || !d_logprobs || !acts || !work || !grads) return RB200_E_NULL;
+  if (!params || !wsplit || !states || !action || !d_logprobs || !acts || !work || !grads) return RB200_E_NULL;
   if (n <= 0) return RB200_E_SHAPE;
   cudaStream_t st = rb::as_stream(stream);
   const int64_t PF = act_floats(n);
@@ -784,15 +651,14 @@ extern "C" int rb200_mlp_backward(const rb200_mlp_layout* L, const float* params
   h.g_mw = G + L->mw; h.g_mb = G + L->mb; h.g_logstd = G + L->logstd; h.g_vw3 = G + L->vw3;
   h.g_b2 = G + L->bb2; h.g_vb2 = G + L->vb2;
   h.n = n; h.act = L->act_dim; h.vdim = L->value_dim;
-  const bool use_h = wsplit && half_mode();
   float* amax = work + 6 * PF;  // 8 floats of the scratch tail: max|dZ3|,|dZ2|,|dZ1| of the policy tower, then the value tower
   float* part = work + 6 * PF + 64;
-  if (use_h) {
+  {
     cudaError_t ce = cudaMemsetAsync(amax, 0, 8 * sizeof(float), st);
     if (ce != cudaSuccess) return (int)ce;
-    h.amax_dz3 = amax;
-    h.amax_dy3 = amax + 3;
   }
+  h.amax_dz3 = amax;
+  h.amax_dy3 = amax + 3;
   const size_t smem = sizeof(float) * ((size_t)2 * (L->act_dim + L->value_dim) * kH + 64 + 2 * kH);
   const bool reg = L->act_dim <= 8 && L->value_dim <= 2;
   if (smem > 48 * 1024) {
@@ -816,54 +682,17 @@ extern "C" int rb200_mlp_backward(const rb200_mlp_layout* L, const float* params
                               {h.g_b2, o + 64, kH}, {h.g_vw3, va, (int64_t)L->value_dim * kH}, {h.g_vb2, o + 64 + kH, kH}};
     if ((e = rb::sum_partials(h.part, grid, row, segs, d_values ? 6 : 4, st))) return e;
   }
-  if (use_h) {
-    TowerIO t[2] = {};
-    t[0].w = tower_w(L, P, false); t[0].wh = tower_wh(L, wsplit, false);
-    t[0].H1 = const_cast<float*>(H1); t[0].H2 = const_cast<float*>(H2); t[0].dZ3 = dZ3; t[0].tA = tA; t[0].tB = tB;
-    t[0].g_w0 = G + L->bw0; t[0].g_b0 = G + L->bb0; t[0].g_w1 = G + L->bw1; t[0].g_b1 = G + L->bb1;
-    t[0].g_w2 = G + L->bw2; t[0].g_b2 = G + L->bb2; t[0].amax = amax;
-    t[1].w = tower_w(L, P, true); t[1].wh = tower_wh(L, wsplit, true);
-    t[1].H1 = const_cast<float*>(G1); t[1].H2 = const_cast<float*>(G2); t[1].dZ3 = dY3; t[1].tA = uA; t[1].tB = uB;
-    t[1].g_w0 = G + L->vw0; t[1].g_b0 = G + L->vb0; t[1].g_w1 = G + L->vw1; t[1].g_b1 = G + L->vb1;
-    t[1].g_w2 = G + L->vw2; t[1].g_b2 = G + L->vb2; t[1].amax = amax + 3;
-    return towers_backward_h(states, idx, n, L->obs_dim, t, d_values ? 2 : 1, part, st);
-  }
-  const TowerWS bws = wsplit ? tower_ws(L, wsplit, false) : TowerWS{};
-  const TowerWS vws = wsplit ? tower_ws(L, wsplit, true) : TowerWS{};
-  if ((e = tower_backward(states, idx, n, L->obs_dim, tower_w(L, P, false), wsplit ? &bws : nullptr, H1, H2,
-                          dZ3, tA, tB, G + L->bw0, G + L->bb0, G + L->bw1, G + L->bb1, G + L->bw2, G + L->bb2, st)))
-    return e;
-  if (d_values &&
-      (e = tower_backward(states, idx, n, L->obs_dim, tower_w(L, P, true), wsplit ? &vws : nullptr, G1, G2,
-                          dY3, uA, uB,
-                          G + L->vw0, G + L->vb0, G + L->vw1, G + L->vb1, G + L->vw2, G + L->vb2, st)))
-    return e;
-  return RB200_OK;
+  TowerIO t[2] = {};
+  t[0].w = tower_w(L, P, false); t[0].wh = tower_wh(L, wsplit, false);
+  t[0].H1 = const_cast<float*>(H1); t[0].H2 = const_cast<float*>(H2); t[0].dZ3 = dZ3; t[0].tA = tA; t[0].tB = tB;
+  t[0].g_w0 = G + L->bw0; t[0].g_b0 = G + L->bb0; t[0].g_w1 = G + L->bw1; t[0].g_b1 = G + L->bb1;
+  t[0].g_w2 = G + L->bw2; t[0].g_b2 = G + L->bb2; t[0].amax = amax;
+  t[1].w = tower_w(L, P, true); t[1].wh = tower_wh(L, wsplit, true);
+  t[1].H1 = const_cast<float*>(G1); t[1].H2 = const_cast<float*>(G2); t[1].dZ3 = dY3; t[1].tA = uA; t[1].tB = uB;
+  t[1].g_w0 = G + L->vw0; t[1].g_b0 = G + L->vb0; t[1].g_w1 = G + L->vw1; t[1].g_b1 = G + L->vb1;
+  t[1].g_w2 = G + L->vw2; t[1].g_b2 = G + L->vb2; t[1].amax = amax + 3;
+  return towers_backward_h(states, idx, n, L->obs_dim, t, d_values ? 2 : 1, part, st);
 }
-
-namespace {
-// Rollout-sized batches (a few thousand rows) give each tower GEMM only n/128 CTAs: the actor and the value tower are
-// independent until the head kernel, so they run concurrently on a forked side stream (fork/join with events; legal
-// inside CUDA-graph capture, where it becomes two parallel branches of the graph).
-struct SideStream {
-  cudaStream_t s = nullptr;
-  cudaEvent_t fork = nullptr, join = nullptr;
-  bool ok = false;
-};
-SideStream& side_stream() {
-  static SideStream ss;
-  static bool tried = false;
-  if (!tried) {
-    tried = true;
-    if (cudaStreamCreateWithFlags(&ss.s, cudaStreamNonBlocking) == cudaSuccess &&
-        cudaEventCreateWithFlags(&ss.fork, cudaEventDisableTiming) == cudaSuccess &&
-        cudaEventCreateWithFlags(&ss.join, cudaEventDisableTiming) == cudaSuccess)
-      ss.ok = true;
-    if (!ss.ok) (void)cudaGetLastError();
-  }
-  return ss;
-}
-}  // namespace
 
 // work: 6 activation tensors; rb200_mlp_fwd_scratch_floats(L, n) floats is always enough
 extern "C" int rb200_mlp_sample(const rb200_mlp_layout* L, const float* params, const float* wsplit,
@@ -872,52 +701,16 @@ extern "C" int rb200_mlp_sample(const rb200_mlp_layout* L, const float* params, 
                                 float* work, rb200_stream_t stream) {
   int e = check_layout(L);
   if (e) return e;
-  if (!params || !states || !action || !logprobs || !work) return RB200_E_NULL;
+  if (!params || !wsplit || !states || !action || !logprobs || !work) return RB200_E_NULL;
   if (n <= 0) return RB200_E_SHAPE;
   cudaStream_t st = rb::as_stream(stream);
   const int64_t PF = act_floats(n);
   float *H1 = work, *H2 = H1 + PF, *H3 = H2 + PF, *G1 = H3 + PF, *G2 = G1 + PF, *G3 = G2 + PF;
   const float* P = params;
-  const TowerWS bws = wsplit ? tower_ws(L, wsplit, false) : TowerWS{};
-  const TowerWS vws = wsplit ? tower_ws(L, wsplit, true) : TowerWS{};
-  const bool use_h = wsplit != nullptr && half_mode();
-  if (use_h) {  // both towers in one grouped launch per layer (no side stream needed)
-    TowerIO t[2] = {};
-    t[0].w = tower_w(L, P, false); t[0].wh = tower_wh(L, wsplit, false); t[0].H1 = H1; t[0].H2 = H2; t[0].H3 = H3;
-    t[1].w = tower_w(L, P, true);  t[1].wh = tower_wh(L, wsplit, true);  t[1].H1 = G1; t[1].H2 = G2; t[1].H3 = G3;
-    if ((e = towers_forward_h(states, nullptr, n, L->obs_dim, t, values ? 2 : 1, st))) return e;
-  }
-  // few tiles per GEMM -> run the two towers side by side
-  const bool fork = !use_h && values != nullptr && wsplit != nullptr && n <= (int64_t)64 * rb::sm_count();
-  SideStream* ss = nullptr;
-  if (fork) {
-    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
-    (void)cudaStreamIsCapturing(st, &cs);
-    static bool created_outside_capture = false;  // never create streams / events while capturing
-    if (cs == cudaStreamCaptureStatusNone || created_outside_capture) {
-      SideStream& r = side_stream();
-      created_outside_capture = true;
-      if (r.ok) ss = &r;
-    }
-  }
-  if (ss) {
-    cudaError_t ce = cudaEventRecord(ss->fork, st);
-    if (ce == cudaSuccess) ce = cudaStreamWaitEvent(ss->s, ss->fork, 0);
-    if (ce != cudaSuccess) return (int)ce;
-    if ((e = tower_forward(states, nullptr, n, L->obs_dim, tower_w(L, P, true), &vws, G1, G2, G3, ss->s))) return e;
-    ce = cudaEventRecord(ss->join, ss->s);
-    if (ce != cudaSuccess) return (int)ce;
-  }
-  if (!use_h && (e = tower_forward(states, nullptr, n, L->obs_dim, tower_w(L, P, false), wsplit ? &bws : nullptr, H1, H2,
-                                   H3, st)))
-    return e;
-  if (ss) {
-    cudaError_t ce = cudaStreamWaitEvent(st, ss->join, 0);
-    if (ce != cudaSuccess) return (int)ce;
-  } else if (!use_h && values && (e = tower_forward(states, nullptr, n, L->obs_dim, tower_w(L, P, true),
-                                          wsplit ? &vws : nullptr, G1, G2, G3, st))) {
-    return e;
-  }
+  TowerIO t[2] = {};  // both towers in one grouped launch per layer
+  t[0].w = tower_w(L, P, false); t[0].wh = tower_wh(L, wsplit, false); t[0].H1 = H1; t[0].H2 = H2; t[0].H3 = H3;
+  t[1].w = tower_w(L, P, true);  t[1].wh = tower_wh(L, wsplit, true);  t[1].H1 = G1; t[1].H2 = G2; t[1].H3 = G3;
+  if ((e = towers_forward_h(states, nullptr, n, L->obs_dim, t, values ? 2 : 1, st))) return e;
   HeadFwdArgs h{};
   h.h3 = H3; h.g3 = values ? G3 : nullptr; h.mw = P + L->mw; h.mb = P + L->mb;
   h.logstd = P + L->logstd; h.vw3 = P + L->vw3; h.noise = noise; h.seed = seed; h.offset = offset;
@@ -954,20 +747,14 @@ extern "C" int rb200_mlp_value(const rb200_mlp_layout* L, const float* params, c
                                const float* states, int64_t n, float* values, float* work, rb200_stream_t stream) {
   int e = check_layout(L);
   if (e) return e;
-  if (!params || !states || !values || !work) return RB200_E_NULL;
+  if (!params || !wsplit || !states || !values || !work) return RB200_E_NULL;
   if (n <= 0 || L->value_dim <= 0) return RB200_E_SHAPE;
   cudaStream_t st = rb::as_stream(stream);
   const int64_t PF = act_floats(n);
   float *G1 = work, *G2 = G1 + PF, *G3 = G2 + PF;
-  const TowerWS vws = wsplit ? tower_ws(L, wsplit, true) : TowerWS{};
-  if (wsplit && half_mode()) {
-    TowerIO t[1] = {};
-    t[0].w = tower_w(L, params, true); t[0].wh = tower_wh(L, wsplit, true); t[0].H1 = G1; t[0].H2 = G2; t[0].H3 = G3;
-    if ((e = towers_forward_h(states, nullptr, n, L->obs_dim, t, 1, st))) return e;
-  } else if ((e = tower_forward(states, nullptr, n, L->obs_dim, tower_w(L, params, true), wsplit ? &vws : nullptr, G1, G2,
-                                G3, st))) {
-    return e;
-  }
+  TowerIO t[1] = {};
+  t[0].w = tower_w(L, params, true); t[0].wh = tower_wh(L, wsplit, true); t[0].H1 = G1; t[0].H2 = G2; t[0].H3 = G3;
+  if ((e = towers_forward_h(states, nullptr, n, L->obs_dim, t, 1, st))) return e;
   value_head_kernel<<<head_grid(n), 256, 0, st>>>(G3, params + L->vw3, values, n, L->value_dim);
   rb::count_launch();
   RB_RETURN_LAUNCH();
@@ -1004,32 +791,17 @@ extern "C" int rb200_mlp_mean(const rb200_mlp_layout* L, const float* params, co
                               int64_t n, float* mean, float* work, rb200_stream_t stream) {
   int e = check_layout(L);
   if (e) return e;
-  if (!params || !states || !mean || !work) return RB200_E_NULL;
+  if (!params || !wsplit || !states || !mean || !work) return RB200_E_NULL;
   if (n <= 0) return RB200_E_SHAPE;
   cudaStream_t st = rb::as_stream(stream);
   const int64_t PF = act_floats(n);
   float *H1 = work, *H2 = H1 + PF, *H3 = H2 + PF;
-  if (wsplit && half_mode()) {
-    TowerIO t[1] = {};
-    t[0].w = tower_w(L, params, false); t[0].wh = tower_wh(L, wsplit, false); t[0].H1 = H1; t[0].H2 = H2; t[0].H3 = H3;
-    if ((e = towers_forward_h(states, nullptr, n, L->obs_dim, t, 1, st))) return e;
-  } else {
-    const TowerWS bws = wsplit ? tower_ws(L, wsplit, false) : TowerWS{};
-    if ((e = tower_forward(states, nullptr, n, L->obs_dim, tower_w(L, params, false), wsplit ? &bws : nullptr, H1, H2,
-                           H3, st)))
-      return e;
-  }
+  TowerIO t[1] = {};
+  t[0].w = tower_w(L, params, false); t[0].wh = tower_wh(L, wsplit, false); t[0].H1 = H1; t[0].H2 = H2; t[0].H3 = H3;
+  if ((e = towers_forward_h(states, nullptr, n, L->obs_dim, t, 1, st))) return e;
   mean_head_kernel<<<head_grid(n), 256, sizeof(float) * (size_t)L->act_dim * kH, st>>>(H3, params + L->mw,
                                                                                       params + L->mb, mean, n,
                                                                                       L->act_dim);
   rb::count_launch();
   RB_RETURN_LAUNCH();
-}
-
-// x -> exact-TF32 (hi, lo) pair (hi + lo ~= x to 2^-22). Lets the caller split the shuffled observations once per
-// iteration instead of once per forward call.
-extern "C" int rb200_split_tf32(const float* x, float* hi, float* lo, int64_t n, rb200_stream_t stream) {
-  if (!x || !hi || !lo) return RB200_E_NULL;
-  if (n <= 0) return RB200_E_SHAPE;
-  return rb::tc::split(x, hi, lo, n, rb::as_stream(stream));
 }

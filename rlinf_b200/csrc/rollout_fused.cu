@@ -20,7 +20,6 @@
 #include <curand_kernel.h>
 
 #include "common.cuh"
-#include "tc_gemm.cuh"  // rb::tc::g_debug_flags (experiment switches)
 
 namespace {
 
@@ -56,13 +55,14 @@ struct FusedArgs {
   float gamma, p_term, noise_std, reward_noise_std;
 };
 
-__device__ __forceinline__ float tanh_fast(float x) {  // same formula as the tensor-core epilogue (tc_gemm.cu)
+__device__ __forceinline__ float tanh_fast(float x) {  // same formula as the tensor-core epilogue (tc_gemm_h.cu)
   const float t = __expf(-2.0f * fabsf(x));
   return copysignf(__fdividef(1.0f - t, 1.0f + t), x);
 }
 
 // out[e][j] = tanh(sum_k in[e][k] * Wt[k][j] + bias[j]) for the CTA's EMAX environment slots; thread j = column j.
 // Wt rows are 1 KB coalesced loads (L2 resident), double-buffered in registers; in[e][k..k+3] are broadcast LDS.128.
+// This one-k-step prefetch and its tiled twin below serve the K that the pipelined layers cannot (K % 16 != 0).
 template <int EMAX>
 __device__ __forceinline__ void layer(const float* __restrict__ in_s, int K, const float* __restrict__ Wt,
                                       const float* __restrict__ bias, float* __restrict__ out_s, int j) {
@@ -138,10 +138,11 @@ __device__ __forceinline__ void layer_tiled(const float* __restrict__ in_s, int 
                     tanh_fast(acc[e].w + b.w));
 }
 
-// ---- deeper software pipelining (the default since round 2; rb200_debug_set_flags bit 1 = round-1 kernels) ----------
+// ---- deeper software pipelining -------------------------------------------------------------------------------------
 // Same arithmetic, same k-ascending fmaf order (bit-identical results), but the weight rows of the next D k-steps
 // are in flight instead of one: with 8 warps / SM the one-k-step prefetch leaves the L2 latency exposed (round 1:
-// 45 us / env step at E = 4 although the FMA work is ~2 us).  Requires K % (4 * D) == 0.
+// 45 us / env step at E = 4 although the FMA work is ~2 us; round 2 with D = 4: 23.1 -> 19.1 ms per 512-step rollout at
+// 512 envs, bit-identical buffers).  Requires K % (4 * D) == 0.
 template <int EMAX, int D>
 __device__ __forceinline__ void layer_pf(const float* __restrict__ in_s, int K, const float* __restrict__ Wt,
                                          const float* __restrict__ bias, float* __restrict__ out_s, int j) {
@@ -224,32 +225,30 @@ __device__ __forceinline__ void layer_tiled_pf(const float* __restrict__ in_s, i
 }
 
 // EMAX == 32 (up to 32 environments per CTA) uses the register-tiled layer, smaller slices the column-per-thread one.
-// PF = weight prefetch depth (0 = the round-1 one-k-step prefetch).
-template <int EMAX, int PF>
+// Weight rows of the next 4 k-steps in flight (2 in the register-tiled layer) when K allows it.
+template <int EMAX>
 __device__ __forceinline__ void layer_any(const float* __restrict__ in_s, int K, const float* __restrict__ Wt,
                                           const float* __restrict__ bias, float* __restrict__ out_s, int j) {
-  if constexpr (PF > 0) {
-    if (K % (4 * PF) == 0) {  // uniform
-      if constexpr (EMAX >= 32) layer_tiled_pf<EMAX, (PF > 2 ? 2 : PF)>(in_s, K, Wt, bias, out_s, j);
-      else layer_pf<EMAX, PF>(in_s, K, Wt, bias, out_s, j);
-      return;
-    }
+  if (K % 16 == 0) {  // uniform
+    if constexpr (EMAX >= 32) layer_tiled_pf<EMAX, 2>(in_s, K, Wt, bias, out_s, j);
+    else layer_pf<EMAX, 4>(in_s, K, Wt, bias, out_s, j);
+    return;
   }
   if constexpr (EMAX >= 32) layer_tiled<EMAX>(in_s, K, Wt, bias, out_s, j);
   else layer<EMAX>(in_s, K, Wt, bias, out_s, j);
 }
 
 // value tower on in_s -> g3 in bufB (uses bufC as the middle buffer); every thread must call it
-template <int EMAX, int PF>
+template <int EMAX>
 __device__ __forceinline__ void value_tower(const FusedArgs& p, const float* in_s, float* bufB, float* bufC, int j) {
   const float* P = p.params;
   const float* wt_v = p.wt;  // value tower first
   const size_t n0 = (size_t)p.obs * kH, nn = (size_t)kH * kH;
-  layer_any<EMAX, PF>(in_s, p.obs, wt_v, P + p.L.vb0, bufB, j);
+  layer_any<EMAX>(in_s, p.obs, wt_v, P + p.L.vb0, bufB, j);
   __syncthreads();
-  layer_any<EMAX, PF>(bufB, kH, wt_v + n0, P + p.L.vb1, bufC, j);
+  layer_any<EMAX>(bufB, kH, wt_v + n0, P + p.L.vb1, bufC, j);
   __syncthreads();
-  layer_any<EMAX, PF>(bufC, kH, wt_v + n0 + nn, P + p.L.vb2, bufB, j);
+  layer_any<EMAX>(bufC, kH, wt_v + n0 + nn, P + p.L.vb2, bufB, j);
   __syncthreads();
 }
 
@@ -264,7 +263,7 @@ __device__ __forceinline__ float value_dot(const float* g3_row, const float* s_v
   return rb::warp_sum(s);
 }
 
-template <int EMAX, int PF>
+template <int EMAX>
 __global__ void __launch_bounds__(kThreads, 1) rollout_fused_kernel(FusedArgs p) {
   extern __shared__ __align__(16) float sm[];
   const int obs = p.obs, act = p.act;
@@ -307,14 +306,14 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_fused_kernel(FusedArgs p)
 
   for (int t = 0; t < T; ++t) {
     // ---- actor tower: x -> bufA -> bufB -> bufA (h3) ----
-    layer_any<EMAX, PF>(x, obs, wt_b, P + p.L.bb0, bufA, j);
+    layer_any<EMAX>(x, obs, wt_b, P + p.L.bb0, bufA, j);
     __syncthreads();
-    layer_any<EMAX, PF>(bufA, kH, wt_b + n0, P + p.L.bb1, bufB, j);
+    layer_any<EMAX>(bufA, kH, wt_b + n0, P + p.L.bb1, bufB, j);
     __syncthreads();
-    layer_any<EMAX, PF>(bufB, kH, wt_b + n0 + nn, P + p.L.bb2, bufA, j);
+    layer_any<EMAX>(bufB, kH, wt_b + n0 + nn, P + p.L.bb2, bufA, j);
     __syncthreads();
     // ---- value tower: x -> bufB -> bufC -> bufB (g3) ----
-    if (has_v) value_tower<EMAX, PF>(p, x, bufB, bufC, j);
+    if (has_v) value_tower<EMAX>(p, x, bufB, bufC, j);
 
     // ---- heads: one warp per environment (head_fwd_kernel, sample mode) ----
     for (int e = warp; e < nE; e += kThreads / 32) {
@@ -433,7 +432,7 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_fused_kernel(FusedArgs p)
       if (j < nE) any = flag_s[j];
       any = __syncthreads_or(any);
       if (any) {
-        value_tower<EMAX, PF>(p, zs, bufB, bufC, j);
+        value_tower<EMAX>(p, zs, bufB, bufC, j);
         for (int e = warp; e < nE; e += kThreads / 32) {
           if (!flag_s[e]) continue;
           const float v = value_dot(bufB + e * kH, s_vw, lane);
@@ -451,7 +450,7 @@ __global__ void __launch_bounds__(kThreads, 1) rollout_fused_kernel(FusedArgs p)
 
   // ---- bootstrap value row T (env_worker.py:1237-1306) ----
   if (has_v) {
-    value_tower<EMAX, PF>(p, x, bufB, bufC, j);
+    value_tower<EMAX>(p, x, bufB, bufC, j);
     for (int e = warp; e < nE; e += kThreads / 32) {
       const float v = value_dot(bufB + e * kH, s_vw, lane);
       if (lane == 0) p.values[(size_t)T * B + e0 + e] = v;
@@ -484,25 +483,17 @@ size_t fused_smem(int obs) {
          sizeof(int) * 2 * EMAX;
 }
 
-template <int EMAX, int PF>
-int launch_fused_pf(const FusedArgs& a, int grid, cudaStream_t st) {
+template <int EMAX>
+int launch_fused(const FusedArgs& a, int grid, cudaStream_t st) {
   const size_t smem = fused_smem<EMAX>(a.obs);
   if (smem > 227 * 1024) return RB200_E_UNSUPPORTED;
-  cudaError_t ce = cudaFuncSetAttribute(rollout_fused_kernel<EMAX, PF>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+  cudaError_t ce = cudaFuncSetAttribute(rollout_fused_kernel<EMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                         (int)smem);
   if (ce != cudaSuccess) return (int)ce;
-  rollout_fused_kernel<EMAX, PF><<<grid, kThreads, smem, st>>>(a);
+  rollout_fused_kernel<EMAX><<<grid, kThreads, smem, st>>>(a);
   rb::count_launch();
   ce = cudaPeekAtLastError();
   return ce == cudaSuccess ? 0 : (int)ce;
-}
-
-template <int EMAX>
-int launch_fused(const FusedArgs& a, int grid, cudaStream_t st) {
-  // default: weight rows of the next 4 k-steps in flight (validated on B200 in round 2: bit-identical buffers for all
-  // four template instances, 23.1 -> 19.1 ms per 512-step rollout at 512 envs); debug bit 1 selects the round-1 kernels
-  if (rb::tc::g_debug_flags & 2) return launch_fused_pf<EMAX, 0>(a, grid, st);
-  return launch_fused_pf<EMAX, 4>(a, grid, st);
 }
 
 }  // namespace

@@ -1,4 +1,4 @@
-// Host-side interface of the tcgen05 3xTF32 GEMMs (tc_gemm.cu).
+// Host-side interface of the fp16-split tcgen05 GEMMs of the MLP towers (tc_gemm_h.cu).
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -10,36 +10,9 @@ constexpr int BM = 128, BN = 256, BK = 32;  // BK fp32 = 128 bytes = one swizzle
 
 enum Epi { EPI_STORE = 0, EPI_BIAS_TANH = 1, EPI_TANHGRAD = 2 };
 
-struct Params {
-  int64_t M;
-  int K;              // multiple of 32
-  const float* bias;  // [256]                         (EPI_BIAS_TANH)
-  const float* h;     // [M,256] previous activation   (EPI_TANHGRAD: out = acc * (1 - h^2))
-  float* c;           // [M,256] fp32 result
-  float* colsum;      // [256] += column sums of the output (bias gradient of the producing layer), or NULL
-  int epi;
-};
-
-// debug/experiment switches (rb200_debug_set_flags): bit 0 = also mask the streamed operand's hi part in shared memory
-// (default off: the tensor core ignores the low 13 mantissa bits of a kind::tf32 operand - verified bit-identical), bit 1 (2) = round-1
-// fused-rollout layers (one-k-step weight prefetch), bit 3 (8) = round-1 3xTF32 GEMMs instead of the fp16-split kernels, bit 5 (32) = one
-// fp16-split GEMM launch per tower, bit 6 (64) = 8 transform warps in the fp16-split forward kernel, bits 8-15 = TF32 kernels' L2
-// prefetch distance in k-blocks (0 = default)
-extern int g_debug_flags;
-
-// C[M,256] = epi( A[M,K] . (B_hi+B_lo)[256,K]^T ).  A is plain fp32 (split into exact-TF32 hi/lo inside the kernel);
-// B is a pre-split weight matrix (rb::tc::split).  All pointers 16-byte aligned.
-int launch(const float* a, const float* b_hi, const float* b_lo, const Params& p, cudaStream_t st);
-// dW[256, IN] += Z[n,256]^T . H[n,IN]   (IN % 32 == 0, <= 256), plain fp32 operands, fp32 atomics into dW
-int wgrad(const float* z, const float* h, float* dW, int64_t n, int IN, cudaStream_t st);
-// x -> (hi, lo) exact-TF32 pair, hi + lo ~= x to 2^-21 relative; hi may alias x.
-int split(const float* x, float* hi, float* lo, int64_t n, cudaStream_t st);
-// out[c][r] = split(x[r][c]) for a small [R,C] matrix
-int split_transpose(const float* x, float* hi, float* lo, int R, int C, cudaStream_t st);
-
 }  // namespace tc
 
-// ---- round 2: fp16-split tensor-core GEMMs (tc_gemm_h.cu), grouped over up to two towers per launch -------------------
+// ---- fp16-split tensor-core GEMMs, grouped over up to two towers per launch ---------------------------------------------
 namespace tch {
 
 struct GemmLaunch {        // one group (tower) of a forward / dgrad launch

@@ -1,13 +1,13 @@
-// K3 tensor-core path, round 2: fp32-accurate GEMMs on tcgen05 `kind::f16` through a 2-way fp16 split.
+// K3 tensor-core path: fp32-accurate GEMMs on tcgen05 `kind::f16` through a 2-way fp16 split.
 //     a = a_hi + a_lo, b = b_hi + b_lo (fp16 numbers, 11 significant bits each; operands pre-scaled by a power of two so
 //     that both halves stay in fp16's normal range);  a.b ~= a_lo.b_hi + a_hi.b_lo + a_hi.b_hi   (dropped a_lo.b_lo ~ 2^-22)
-// Same three-MMA compensation as the round-1 3xTF32 kernels (tc_gemm.cu) with the same 2^-22 truncation, but
+// This is the three-MMA compensation of a 3xTF32 GEMM with the same 2^-22 truncation, but
 //   * kind::f16 issues at twice the kind::tf32 rate, so an fp32-accurate product costs peak/3 instead of peak/6;
 //   * operands are 2 bytes in shared memory: the three MMAs re-read 72 KB per 128x256x32 k-block instead of 147 KB and
-//     the weight tiles TMA-fill 32 KB instead of 64 KB (round 1 was bound by exactly this shared-memory traffic);
+//     the weight tiles TMA-fill 32 KB instead of 64 KB (a 3xTF32 version, measured in round 1, was bound by exactly this
+//     shared-memory traffic);
 //   * the weights are packed per k-block as pre-swizzled fp16 (hi | lo) tiles - a K-major forward pack and an MN-major dgrad
-//     pack per matrix, written by one pack kernel - and fetched with ONE 32 KB bulk copy per k-block; the transposed fp32
-//     weight copies of round 1 and their 8 refresh kernels are gone;
+//     pack per matrix, written by one pack kernel - and fetched with ONE 32 KB bulk copy per k-block;
 //   * one launch serves BOTH towers (policy backbone + value MLP have identical shapes): grouped tile scheduling halves
 //     the launches and fills the tail wave of small per-rank batches.
 // Activations / activation gradients stay plain fp32 in HBM (one copy); the streamed operand is TMA-landed as fp32
@@ -44,15 +44,16 @@ constexpr int kB16 = BN * BK * 2;   // 16 KB per fp16 half of the weight tile
 constexpr int kOpBytes = 2 * kA16;  // 16 KB: A hi | A lo
 constexpr int kWBytes = 2 * kB16;   // 32 KB: W hi | W lo
 constexpr int kRingBytes = kAStages * kA32 + kBStages * kOpBytes + kWStages * kWBytes;  // 64 + 32 + 96 = 192 KB
-constexpr int kXfWarpsDefault = 4;  // transform warps per CTA: template parameter XF of the forward / dgrad kernel (4 or 8)
+constexpr int kXfWarps = 4;   // transform warps of the forward / dgrad kernel, one per scheduler (8 measured no faster:
+                              // DESIGN.md section 4)
 constexpr int kEpiWarps = 8;  // two per TMEM lane quarter, 128 of the 256 output columns each: the bias+tanh / (1-h^2)
                               // epilogue of one warp per scheduler took 7.8 k cycles per tile against 6.1 k of MMA
-constexpr int threads_for(int xf) { return 32 * (2 + xf + kEpiWarps); }  // producer, MMA, transform, epilogue
+constexpr int kThreads = 32 * (2 + kXfWarps + kEpiWarps);  // producer, MMA, transform, epilogue
 constexpr int kStagingBytes = kEpiWarps * 4096;  // one [32 x 32] fp32 staging tile per epilogue warp
 constexpr int kTmemCols = 512;
 constexpr int kWeightScaleLog2 = 10;  // weights are stored as fp16 (hi, lo) of w * 2^10 (|w| <~ 1: both halves normal)
 
-// ---- PTX wrappers (same instructions as tc_gemm.cu) ---------------------------------------------------------------
+// ---- PTX wrappers -----------------------------------------------------------------------------------------------
 __device__ __forceinline__ void tmem_alloc(uint32_t* smem_dst, uint32_t ncols) {
   asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tma::smem_u32(smem_dst)),
                "r"(ncols)
@@ -210,14 +211,12 @@ struct GemmParams {
   int epi;
   int b_mn;  // 0: weights K-major (forward), 1: MN-major (dgrad: B(n = in, k = out) = W[out][in])
   int ngroups;
-  int flags;
   float* part;      // [CTAs per group][ngroups][256] column sums (EPI_TANHGRAD with colsum)
   long long* prof;  // [16] (PROF instantiation only)
 };
 
-template <bool PROF, int kXfWarps>
-__global__ void __launch_bounds__(threads_for(kXfWarps), 1) tc_h_gemm_kernel(const __grid_constant__ GemmParams P) {
-  constexpr int kThreads = threads_for(kXfWarps);
+template <bool PROF>
+__global__ void __launch_bounds__(kThreads, 1) tc_h_gemm_kernel(const __grid_constant__ GemmParams P) {
   long long pc[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
   const long long t_start = PROF ? clock64() : 0;
   extern __shared__ uint8_t smem_raw[];
@@ -509,7 +508,7 @@ struct WgradParams {
   float* part;             // [chunks][ngroups][256 * IN] partial dW of each sample chunk
   const float* amax_z[2];  // max|dZ| per group (or NULL)
   int64_t n;
-  int IN, kb_per_chunk, ngroups, flags;
+  int IN, kb_per_chunk, ngroups;
   long long* prof;  // [16] (PROF instantiation: slots 9..15)
 };
 
@@ -744,13 +743,9 @@ int launch(const GemmLaunch* L, int ngroups, int64_t M, int K, int epi, int b_mn
   if (ngroups < 1 || ngroups > 2 || K % BK != 0 || K <= 0 || M <= 0) return RB200_E_SHAPE;
   // Two towers in one launch: measured on B200 (profiles/r02_tc_h_gemm_grouping.txt) grouped is never slower than one
   // launch per tower (1.18 vs 1.21 ms per 6-GEMM forward at 262144 rows, 0.21 vs 0.24 ms at 32768 where it fills the
-  // tail wave).  Debug flag 32 forces one launch per tower.
-  if (ngroups == 2 && (rb::tc::g_debug_flags & 32)) {
-    int e = launch(L, 1, M, K, epi, b_mn, part, st);
-    return e ? e : launch(L + 1, 1, M, K, epi, b_mn, part, st);
-  }
+  // tail wave).
   GemmParams P{};
-  P.M = M; P.K = K; P.epi = epi; P.b_mn = b_mn; P.ngroups = ngroups; P.flags = rb::tc::g_debug_flags;
+  P.M = M; P.K = K; P.epi = epi; P.b_mn = b_mn; P.ngroups = ngroups;
   for (int g = 0; g < ngroups; ++g) {
     const GemmLaunch& l = L[g];
     const uintptr_t al = reinterpret_cast<uintptr_t>(l.a) | reinterpret_cast<uintptr_t>(l.b_hi) |
@@ -766,11 +761,9 @@ int launch(const GemmLaunch* L, int ngroups, int64_t M, int K, int epi, int b_mn
   constexpr int kSmem = kRingBytes + kStagingBytes + 1024 + (int)sizeof(Barriers);
   static_assert(kSmem <= 232448, "tc_h_gemm_kernel shared memory");
   if (!attr_done) {
-    cudaError_t ce = cudaFuncSetAttribute(tc_h_gemm_kernel<false, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
+    cudaError_t ce = cudaFuncSetAttribute(tc_h_gemm_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
     if (ce == cudaSuccess)
-      ce = cudaFuncSetAttribute(tc_h_gemm_kernel<false, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
-    if (ce == cudaSuccess)
-      ce = cudaFuncSetAttribute(tc_h_gemm_kernel<true, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
+      ce = cudaFuncSetAttribute(tc_h_gemm_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
     if (ce != cudaSuccess) return (int)ce;
     attr_done = true;
   }
@@ -785,11 +778,8 @@ int launch(const GemmLaunch* L, int ngroups, int64_t M, int K, int epi, int b_mn
     if (part == nullptr) return RB200_E_NULL;
     P.part = part;
   }
-  // transform warps: 4 (one per scheduler) or 8 (debug flag 64) - see DESIGN.md section 4
-  const bool xf8 = ((rb::tc::g_debug_flags & 64) != 0) != (kXfWarpsDefault == 8);
-  if (g_prof) tc_h_gemm_kernel<true, 4><<<per_group * ngroups, threads_for(4), kSmem, st>>>(P);
-  else if (xf8) tc_h_gemm_kernel<false, 8><<<per_group * ngroups, threads_for(8), kSmem, st>>>(P);
-  else tc_h_gemm_kernel<false, 4><<<per_group * ngroups, threads_for(4), kSmem, st>>>(P);
+  if (g_prof) tc_h_gemm_kernel<true><<<per_group * ngroups, kThreads, kSmem, st>>>(P);
+  else tc_h_gemm_kernel<false><<<per_group * ngroups, kThreads, kSmem, st>>>(P);
   rb::count_launch();
   cudaError_t ce = cudaPeekAtLastError();
   if (ce != cudaSuccess || nseg == 0) return (int)ce;
@@ -799,7 +789,7 @@ int launch(const GemmLaunch* L, int ngroups, int64_t M, int K, int epi, int b_mn
 int wgrad(const WgradLaunch* L, int ngroups, int64_t n, int IN, float* part, cudaStream_t st) {
   if (ngroups < 1 || ngroups > 2 || n <= 0 || IN <= 0 || IN > 256 || IN % 32 != 0) return RB200_E_SHAPE;
   WgradParams P{};
-  P.n = n; P.IN = IN; P.ngroups = ngroups; P.flags = rb::tc::g_debug_flags;
+  P.n = n; P.IN = IN; P.ngroups = ngroups;
   for (int g = 0; g < ngroups; ++g) {
     const uintptr_t al = reinterpret_cast<uintptr_t>(L[g].z) | reinterpret_cast<uintptr_t>(L[g].h) |
                          reinterpret_cast<uintptr_t>(L[g].dW);

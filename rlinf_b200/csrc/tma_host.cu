@@ -38,10 +38,9 @@ int encode_tmap_2d(CUtensorMap* out, const void* base, int elem_bytes, uint64_t 
 }
 
 
-namespace tc {
-// [rows, cols] fp32 row-major, box [box_rows x 32 floats] (128 bytes inner = one SWIZZLE_128B span)
-static int encode_swz(CUtensorMap* out, const float* base, uint64_t rows, uint64_t cols, uint32_t box_rows,
-                      CUtensorMapSwizzle swz) {
+namespace tch {
+// fp32 [rows, cols] row-major, box [box_rows x 32 floats], SWIZZLE_128B (landing tiles of the fp16-split kernels)
+int encode_f32_sw128(CUtensorMap* out, const float* base, uint64_t rows, uint64_t cols, uint32_t box_rows) {
   auto enc = get_encode();
   if (!enc) return -1;
   cuuint64_t gdim[2] = {cols, rows};
@@ -49,24 +48,9 @@ static int encode_swz(CUtensorMap* out, const float* base, uint64_t rows, uint64
   cuuint32_t box[2] = {32u, box_rows};
   cuuint32_t estr[2] = {1, 1};
   CUresult r = enc(out, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(base), gdim, gstride, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   return r == CUDA_SUCCESS ? 0 : (int)r;
-}
-int encode_sw128(CUtensorMap* out, const float* base, uint64_t rows, uint64_t cols, uint32_t box_rows) {
-  return encode_swz(out, base, rows, cols, box_rows, CU_TENSOR_MAP_SWIZZLE_128B);
-}
-// box [32 rows x 32 floats] = one 4 KB group of the MN-major operand tiles of the wgrad GEMM. MN-major TF32 operands
-// must use the 128B-span / 32B-atom swizzle (UMMA LayoutType::SWIZZLE_128B_BASE32B; cutlass sm100_common.inl:92).
-int encode_sw128_box32(CUtensorMap* out, const float* base, uint64_t rows, uint64_t cols) {
-  return encode_swz(out, base, rows, cols, 32, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B);
-}
-}  // namespace tc
-
-namespace tch {
-// fp32 [rows, cols] row-major, box [box_rows x 32 floats], SWIZZLE_128B (landing tiles of the fp16-split kernels)
-int encode_f32_sw128(CUtensorMap* out, const float* base, uint64_t rows, uint64_t cols, uint32_t box_rows) {
-  return tc::encode_sw128(out, base, rows, cols, box_rows);
 }
 // fp16 [rows, cols] row-major, box [box_rows x box_cols], SWIZZLE_64B / SWIZZLE_128B (pre-split weight copies)
 int encode_f16(CUtensorMap* out, const void* base, uint64_t rows, uint64_t cols, uint32_t box_cols, uint32_t box_rows,

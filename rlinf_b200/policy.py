@@ -39,8 +39,7 @@ class MLPPolicy:
         self.flat_grads = torch.zeros(n, dtype=torch.float32, device=self.device)
         self._spec = self._build_spec()
         self._scratch: dict[tuple, torch.Tensor] = {}
-        # tensor-core operand cache (packed fp16 hi/lo tiles of the hidden-layer weights; TF32 copies with debug flag 8)
-        self.use_tensor_cores = True
+        # tensor-core operand cache (packed fp16 hi/lo tiles of the hidden-layer weights)
         self.wsplit = torch.zeros(int(lib.rb200_mlp_wsplit_floats(C.byref(self.layout))), dtype=torch.float32,
                                   device=self.device)
         self._wsplit_fresh = False
@@ -82,9 +81,7 @@ class MLPPolicy:
         self._wsplit_fresh = False
 
     def _ws(self):
-        """Pointer to an up-to-date weight split (refreshed lazily, 20 tiny kernels), or NULL."""
-        if not self.use_tensor_cores:
-            return None
+        """Pointer to an up-to-date weight split (refreshed lazily, one launch)."""
         if not self._wsplit_fresh:
             L.check(L.load().rb200_mlp_prepare_weights(C.byref(self.layout), L.ptr(self.flat_params),
                                                        L.ptr(self.wsplit), L.stream_ptr()), "mlp_prepare_weights")

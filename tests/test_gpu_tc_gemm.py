@@ -1,53 +1,10 @@
-"""tcgen05 3xTF32 GEMM building block vs an fp64 matmul (GPU)."""
+"""fp16-split tcgen05 GEMM building blocks of the MLP towers vs an fp64 matmul (GPU)."""
 import pytest
 import torch
 
 pytestmark = pytest.mark.gpu
 
 
-@pytest.mark.parametrize("M,K", [(128, 32), (128, 256), (1000, 128), (5000, 256), (262144, 256)])
-def test_tc_gemm_matches_fp64(M, K):
-    from rlinf_b200 import _lib as L
-
-    lib = L.load()
-    g = torch.Generator(device="cuda").manual_seed(M + K)
-    A = torch.randn(M, K, device="cuda", generator=g)
-    B = torch.randn(256, K, device="cuda", generator=g) / K ** 0.5
-    C = torch.empty(M, 256, device="cuda")
-    work = torch.empty(2 * M * K + 512 * K, device="cuda")
-    L.check(lib.rb200_tc_gemm(L.ptr(A), L.ptr(B), L.ptr(C), M, K, L.ptr(work), L.stream_ptr()), "tc_gemm")
-    torch.cuda.synchronize()
-    n = min(M, 4096)
-    ref = (A[:n].double() @ B.double().T)
-    err = (C[:n].double() - ref).abs().max().item()
-    scale = ref.abs().max().item()
-    # fp32-level accuracy (plain TF32 would be ~1e-3 relative)
-    assert err <= 5e-6 * scale + 1e-6, (err, scale)
-    if M > n:  # spot-check the tail rows too
-        ref2 = (A[-256:].double() @ B.double().T)
-        assert (C[-256:].double() - ref2).abs().max().item() <= 5e-6 * scale + 1e-6
-
-
-@pytest.mark.parametrize("n,IN", [(32, 32), (1000, 128), (4096, 256), (70000, 256), (262144, 128)])
-def test_tc_wgrad_matches_fp64(n, IN):
-    from rlinf_b200 import _lib as L
-
-    lib = L.load()
-    g = torch.Generator(device="cuda").manual_seed(n + IN)
-    Z = torch.randn(n, 256, device="cuda", generator=g) / n ** 0.5
-    H = torch.randn(n, IN, device="cuda", generator=g)
-    dW = torch.ones(256, IN, device="cuda")  # accumulates (+=)
-    work = torch.empty(2 * n * (256 + IN), device="cuda")
-    L.check(lib.rb200_tc_wgrad(L.ptr(Z), L.ptr(H), L.ptr(dW), n, IN, L.ptr(work), L.stream_ptr()), "tc_wgrad")
-    torch.cuda.synchronize()
-    ref = 1.0 + Z.double().T @ H.double()
-    err = (dW.double() - ref).abs().max().item()
-    scale = (ref - 1.0).abs().max().item()
-    # fp32 accumulation over n samples (TMEM accumulators are fp32, like any fp32 GEMM): error grows ~sqrt(n)
-    assert err <= (5e-6 + 2e-7 * n ** 0.5) * scale + 2e-6, (err, scale)
-
-
-# ---- round 2: fp16-split kind::f16 kernels (csrc/tc_gemm_h.cu) ------------------------------------------------------------
 def _amax(t):
     return t.abs().max().reshape(1).to(torch.float32)
 
@@ -108,9 +65,9 @@ def test_tc_wgrad_h_matches_fp64(n, IN, grad_like):
     assert err < 2e-6, err
 
 
-def test_tc_h_kernel_timing_report():
-    """Not an assertion on speed: prints per-launch times of the round-1 3xTF32 and the round-2 fp16-split kernels at
-    the headline mini-batch shape so that every GPU test log carries them."""
+def test_fp16_split_kernel_timing_report():
+    """Not an assertion on speed: prints per-launch times of the fp16-split kernels at the headline mini-batch shape so
+    that every GPU test log carries them."""
     from rlinf_b200 import _lib as L
 
     lib = L.load()
@@ -134,10 +91,8 @@ def test_tc_h_kernel_timing_report():
         return e0.elapsed_time(e1) / reps * 1e3
 
     t = {
-        "tf32x3 gemm": timeit(lambda: lib.rb200_tc_gemm(L.ptr(A), L.ptr(B), L.ptr(C), n, K, L.ptr(work), L.stream_ptr())),
         "f16x2 gemm fwd": timeit(lambda: lib.rb200_tc_gemm_h(L.ptr(A), L.ptr(B), L.ptr(C), n, K, 0, None, L.ptr(work), L.stream_ptr())),
         "f16x2 gemm dgrad": timeit(lambda: lib.rb200_tc_gemm_h(L.ptr(A), L.ptr(B), L.ptr(C), n, K, 1, None, L.ptr(work), L.stream_ptr())),
-        "tf32x3 wgrad": timeit(lambda: lib.rb200_tc_wgrad(L.ptr(C), L.ptr(A), L.ptr(dW), n, K, None, L.stream_ptr())),
         "f16x2 wgrad": timeit(lambda: lib.rb200_tc_wgrad_h(L.ptr(C), L.ptr(A), L.ptr(dW), n, K, None, L.stream_ptr())),
     }
     print("TIMING us/launch (incl. the weight-split helper kernel of the test entries):", {k: round(v, 1) for k, v in t.items()})

@@ -6,14 +6,10 @@ n = int(sys.argv[1]) if len(sys.argv) > 1 else 262144
 pol = MLPPolicy(obs_dim=128, action_dim=8, seed=0)
 states = torch.randn(n, 128, device='cuda'); action = torch.randn(n, 8, device='cuda')
 dl = torch.randn(n, 8, device='cuda') / n; dv = torch.randn(n, 1, device='cuda') / n
-modes = (True,) if len(sys.argv) > 2 else (True, False)
-for tc in modes:
-    pol.use_tensor_cores = tc
-    pol.mark_params_changed()
-    for _ in range(2):
-        out = pol.forward_train(states, action, compute_entropy=False); pol.backward(dl, dv, None)
-    torch.cuda.synchronize()
-    e = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
-    e[0].record(); out = pol.forward_train(states, action, compute_entropy=False); e[1].record(); pol.backward(dl, dv, None); e[2].record()
-    torch.cuda.synchronize()
-    print(f"tensor_cores={tc} n={n}: fwd {e[0].elapsed_time(e[1]):.3f} ms  bwd {e[1].elapsed_time(e[2]):.3f} ms", flush=True)
+for _ in range(2):
+    out = pol.forward_train(states, action, compute_entropy=False); pol.backward(dl, dv, None)
+torch.cuda.synchronize()
+e = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
+e[0].record(); out = pol.forward_train(states, action, compute_entropy=False); e[1].record(); pol.backward(dl, dv, None); e[2].record()
+torch.cuda.synchronize()
+print(f"n={n}: fwd {e[0].elapsed_time(e[1]):.3f} ms  bwd {e[1].elapsed_time(e[2]):.3f} ms", flush=True)
